@@ -224,7 +224,12 @@ def main():
                     help="'score' = the headline metric (+ sustained + train sub-records); 'train' = only the training record "
                          "(fwd+bwd(+DDP all-reduce)+clip+Adam step, samples/s) as the line; 'train_tokens' = the same step from "
                          "TOKEN tensors, MSA news encoder included (reference Model.forward, model.py:54-77), eager, one GPU")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="score mode: write the click logits of the last timed step to DIR/logits.npy (float32; "
+                         "DIR/logits_rank<r>.npy per rank when N>1), to compare two builds on identical seeded inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'ours' or args.mode != 'score'):
+        ap.error('--dump-outputs needs --impl ours --mode score')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     if args.impl == 'reference':
@@ -313,13 +318,18 @@ def run_score(args, rank, local_rank, world, dev):
     # the public pipelined driver: the flag kernels of batch k+1 are enqueued ahead of the encoder pass of batch k and
     # the host waits for their counts (the only synchronisation of a step) while that pass runs
     step_events = []
-    scoring.score_resident_batches(scorer, index_batches(args.warmup, total_steps), events=step_events)
+    outs = scoring.score_resident_batches(scorer, index_batches(args.warmup, total_steps), events=step_events)
     e1.record()
     if profile_range:
         torch.cuda.synchronize()
         torch.cuda.cudart().cudaProfilerStop()
     barrier()
     launches = _lib.launch_count()
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'logits.npy' if world == 1 else 'logits_rank%d.npy' % rank),
+                outs[-1].cpu().numpy())
+    del outs
     ms_resident = _max_over_ranks(e0.elapsed_time(e1), world, dev)
     marks = [e0] + step_events
     step_ms = sorted(marks[k].elapsed_time(marks[k + 1]) for k in range(len(marks) - 1))

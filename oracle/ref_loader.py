@@ -1,7 +1,8 @@
-"""TEST INFRASTRUCTURE ONLY -- import the UNMODIFIED reference modules from /root/reference (this container only).
+"""TEST INFRASTRUCTURE ONLY -- import the UNMODIFIED reference modules from a checkout of the original DIGAT code, which
+is not part of this repository: set ``DIGAT_REFERENCE_ROOT`` to its directory.
 
-The reference cannot travel to the GPU box (/root/reference does not exist there), so this loader is used only
-by ``oracle/make_golden.py`` (fixture generation) and by CPU tests that skip when the reference is absent.
+This loader is used only by ``oracle/make_golden.py`` (fixture generation) and by the CPU tests of
+``tests/test_reference_dropin.py``, which skip when no reference checkout is given.
 
 Three modules the reference imports are not installed and there is no network (SURVEY.md section 8c):
 ``torchtext`` (MIND_corpus.py:8), ``sentence_transformers`` (construct_SAG.py:4) -- both off the hot path, stubbed
@@ -11,17 +12,17 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get('DIGAT_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('DIGAT_REFERENCE_ROOT', '')
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, 'graphEncoders.py'))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, 'graphEncoders.py'))
 
 
 def load_reference():
     """Returns the reference's (graphEncoders, layers, model, evaluate) modules."""
     if not reference_available():
-        raise RuntimeError('reference tree not found at ' + REFERENCE_ROOT)
+        raise RuntimeError('reference tree not found: set DIGAT_REFERENCE_ROOT to a checkout of the original DIGAT code')
     from . import scatter_shim
     if 'torchtext' not in sys.modules:
         tt = types.ModuleType('torchtext')
@@ -43,6 +44,6 @@ def load_reference():
         sys.path.append(REFERENCE_ROOT)
     import importlib
     # the reference modules import each other by bare name (``from layers import ...``), so they are imported
-    # through the normal machinery with /root/reference appended (not prepended) to sys.path
+    # through the normal machinery with the reference root appended (not prepended) to sys.path
     mods = {name: importlib.import_module(name) for name in ('layers', 'graphEncoders', 'evaluate', 'construct_SAG')}
     return mods['graphEncoders'], mods['layers'], mods['evaluate'], mods['construct_SAG']

@@ -24,7 +24,7 @@ def sha(a):
 
 
 def case_inputs(name):
-    """Same construction as oracle/make_golden.py::case_inputs (kept separate: tests must not need /root/reference)."""
+    """Same construction as oracle/make_golden.py::case_inputs (kept separate: tests must not need the reference code)."""
     N, hops, L, rows, keep, scale = CASES[name]
     cfg = synth.make_config(SAG_neighbors=N, SAG_hops=hops, graph_depth=L)
     sd = synth.make_state_dict(cfg, seed=11)

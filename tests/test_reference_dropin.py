@@ -1,8 +1,9 @@
 """The "one import line" claim of INTEGRATION.md, executed: the UNMODIFIED reference ``model.py`` is imported with
 ``graphEncoders`` resolved to ``digat_b200.graphEncoders`` and driven through ``Model.__init__`` (string dispatch,
 model.py:18-31), ``load_state_dict`` of a checkpoint written by the reference's own encoder (main.py:23,36) and the argument
-plumbing of ``Model.inference`` / ``Model.forward`` (model.py:54-90).  Runs where /root/reference exists (this container);
-no kernel is launched (no GPU here) -- the numerical side of the same loop is tests/test_gpu_dropin.py."""
+plumbing of ``Model.inference`` / ``Model.forward`` (model.py:54-90).  The reference code is not part of this repository:
+these tests run when DIGAT_REFERENCE_ROOT names a checkout of it and skip otherwise.  No kernel is launched -- the
+numerical side of the same loop is tests/test_gpu_dropin.py."""
 import importlib.util
 import os
 import sys
@@ -13,7 +14,7 @@ import torch
 
 from oracle.ref_loader import REFERENCE_ROOT, load_reference, reference_available
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason='/root/reference not present on this box')
+pytestmark = pytest.mark.skipif(not reference_available(), reason='needs the original DIGAT code: set DIGAT_REFERENCE_ROOT')
 
 ENCODERS = ['DIGAT', 'wo_SA', 'Seq_SA', 'wo_interaction', 'news_graph_wo_inter', 'user_graph_wo_inter']
 
