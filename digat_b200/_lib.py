@@ -21,6 +21,8 @@ SIGNATURES = {
     'digat_split_bf16': [c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
     'digat_linear_tf32_bf16c': [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
                                 c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    'digat_linear_bf16': [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+                          c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     'digat_linear_tf32x3_splitk': [c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                    c_int64, c_void_p],
     'digat_debug_set_gemm_variant': [c_int],

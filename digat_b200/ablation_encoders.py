@@ -99,6 +99,8 @@ class _AblationEncoder(DIGAT):
     # ---------------------------------------------------------------------------------- packed weights
     def _weights(self):
         """Kernel-side layout of whatever this variant owns (same conventions as DIGAT._weights)."""
+        if self._bf16_projections():
+            raise RuntimeError("%s: projection_precision = 'bf16' is implemented for DIGAT only" % type(self).__name__)
         params = list(self.parameters())
         key = tuple((p.data_ptr(), p._version) for p in params)
         if self._packed is not None and key == self._packed_key:

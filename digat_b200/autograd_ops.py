@@ -464,7 +464,8 @@ def encode_with_grad(enc, Xn, An, Mn, Xh, Au, Mc, ci, schedule='digat'):
     """Reference DIGAT.forward (graphEncoders.py:177-187) with autograd; dropout active iff enc.training.
     schedule: 'digat' (the dual-graph schedule), or one of the two ablations built from the same pieces --
     'wo_SA' (graphEncoders.py:277-284: the candidate's own embedding drives L user layers, one user context at the end) and
-    'Seq_SA' (:388-396: a fixed news-sequence context, user layers and contexts as DIGAT)."""
+    'Seq_SA' (:388-396: a fixed news-sequence context, user layers and contexts as DIGAT).
+    Every GEMM here is fp32 (3xTF32 or exact): enc.projection_precision applies to the no-grad inference paths only."""
     D, L, H, S = enc.news_embedding_dim, enc.graph_depth, enc.max_history_num, enc.category_num
     p = enc.dropout_rate if enc.training else 0.0
     B = Xn.shape[0]

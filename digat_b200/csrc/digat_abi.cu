@@ -6,6 +6,7 @@
 #include "gemm_tcgen05.cuh"
 #include "gemm_tcgen05_pair.cuh"
 #include "gemm_tcgen05_persistent.cuh"
+#include "gemm_bf16.cuh"
 #include "pair_attention.cuh"
 #include "pair_attention_sparse.cuh"
 #include "context.cuh"
@@ -105,6 +106,14 @@ int digat_linear_tf32_bf16c(const float* A, int lda, const float* W_hi, const vo
     if (N % 240 == 0)
         return launch_tf32x3_persistent<240>(A, lda, W_hi, nullptr, ldw, bias, C, ldc, M, N, K, gb, as_stream(stream), W_hb, W_lb);
     return launch_tf32x3_persistent<208>(A, lda, W_hi, nullptr, ldw, bias, C, ldc, M, N, K, gb, as_stream(stream), W_hb, W_lb);
+}
+
+int digat_linear_bf16(const float* A, int lda, const void* W_b, int ldw, const float* bias, float* C, int ldc,
+                      int M, int N, int K, const float* group_bias, int group_rows, int group_col0, int group_cols,
+                      int group_ld, const int32_t* c_row_index, void* stream) {
+    return launch_linear_bf16(A, lda, W_b, ldw, bias, C, ldc, M, N, K,
+                              GroupBias{group_bias, group_rows, group_col0, group_cols, group_ld, c_row_index},
+                              as_stream(stream));
 }
 
 int digat_debug_set_layer_mode(int mode) {

@@ -47,21 +47,26 @@ constexpr int kTcEpiWarps = 8;                  // two epilogue warps per TMEM l
 constexpr int kTcPersistThreads = (2 + 4 + kTcEpiWarps) * 32;
 
 // kCl: 1 = independent CTAs; 2 = W multicast across a CTA pair (experiment); 3 = 2-CTA MMA (cta_group::2, M = 256): each
-// CTA of the pair loads and holds only HALF of the W tile, the leader CTA issues the MMAs for both
-template <int BN, int kCl = 1>
+// CTA of the pair loads and holds only HALF of the W tile, the leader CTA issues the MMAs for both.
+// kOne: the plain BF16 GEMM (gemm_bf16.cuh): a stage holds the raw fp32 A tile, bf16(A) and ONE bf16 plane of W.
+template <int BN, int kCl = 1, bool kOne = false>
 struct TcPersistCfg {
     static constexpr int A_BYTES = 128 * kTcBK * 4;
     static constexpr int W_ROWS = kCl == 3 ? BN / 2 : BN;                // W rows resident in this CTA's shared memory
     static constexpr int W_BYTES = W_ROWS * kTcBK * 4;
-    static constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * W_BYTES;
+    static constexpr int STAGE_BYTES = kOne ? A_BYTES + A_BYTES / 2 + W_BYTES / 2 : 2 * A_BYTES + 2 * W_BYTES;
+    static constexpr int ACC_BUFS = kOne ? 2 : 1;                        // TMEM accumulator buffers (tiles in flight)
     static constexpr int MAX_N = 1280;                                   // bias vector kept in smem for the whole N
     static constexpr int GB_GROUPS = 16;                                 // row groups of one 128-row tile staged in smem
     static constexpr int EXTRA = 512 /*barriers*/ + MAX_N * 4 + kTcEpiWarps * 32 * 20 * 4 /*epilogue staging*/ + GB_GROUPS * BN * 4;
-    static constexpr int STAGES = (226 * 1024 - EXTRA) / STAGE_BYTES > 6 ? 6 : (226 * 1024 - EXTRA) / STAGE_BYTES;
+    static constexpr int MAX_STAGES = kOne ? 8 : 6;
+    static constexpr int STAGES = (226 * 1024 - EXTRA) / STAGE_BYTES > MAX_STAGES ? MAX_STAGES : (226 * 1024 - EXTRA) / STAGE_BYTES;
     static constexpr int TMEM_COLS = 2 * BN <= 256 ? 256 : 512;
     static constexpr size_t SMEM = (size_t)STAGES * STAGE_BYTES + EXTRA;
     static_assert(STAGES >= 3, "not enough shared memory for the pipeline");
-    static_assert(A_BYTES % 512 == 0 && W_BYTES % 512 == 0, "operand tiles must start on a swizzle-atom boundary");
+    static_assert(A_BYTES % 512 == 0 && W_BYTES % 512 == 0 && STAGE_BYTES % 512 == 0,
+                  "operand tiles must start on a swizzle-atom boundary");
+    static_assert(!kOne || (kCl == 1 && 2 * BN <= 512), "the BF16 GEMM keeps two accumulators of one CTA in TMEM");
 };
 
 // kBf16: the TF32+BF16 scheme.  The two correction products are ~2^-11 of the result, so they only need ~9 good bits:
@@ -70,22 +75,27 @@ struct TcPersistCfg {
 // truncation error).  bf16 MMAs run at twice the TF32 rate: per 16-wide k-block the tensor pipe does 2 TF32 MMAs + 2 BF16
 // MMAs = 4 TF32-MMA times instead of 6.  The stage keeps its size: A_lo (tf32) becomes two bf16 tiles of half the size,
 // W_lo (tf32) becomes the two bf16 planes of W (map_w2 = bf16(W_hi), map_w3 = bf16(W_lo); SWIZZLE_32B tiles).
-template <int BN, bool kBf16, int kCl>
+//
+// kOne: C = bf16_rn(A) * W_b^T, one kind::f16 MMA (K = 16) per k-block into ONE accumulator (map_whi = W_b, SWIZZLE_32B;
+// the other maps are unused).  The transform warps write bf16_rn(A) (the A_hi-free half of the kBf16 transform).  Two
+// accumulator buffers alternate between tiles: the MMA warp fills buffer (j+1)&1 while the epilogue drains buffer j&1.
+// The epilogue is the same code as the fp32 schemes' (bias, row-group bias, row scatter, staged row-segment stores).
+template <int BN, bool kBf16, int kCl, bool kOne = false>
 __global__ void __launch_bounds__(kTcPersistThreads, 1)
 gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_whi,
                               const __grid_constant__ CUtensorMap map_wlo, const __grid_constant__ CUtensorMap map_w3,
                               const float* __restrict__ bias,
                               float* __restrict__ C, int ldc, int M, int N, int K, GroupBias gb) {
-    using Cfg = TcPersistCfg<BN, kCl>;
+    using Cfg = TcPersistCfg<BN, kCl, kOne>;
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = smem_raw;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)Cfg::STAGES * Cfg::STAGE_BYTES);
     uint64_t* full = bars;                                  // [STAGES] TMA bytes landed
     uint64_t* ready = bars + Cfg::STAGES;                   // [STAGES] A_lo written by the transform warps
     uint64_t* empty = bars + 2 * Cfg::STAGES;               // [STAGES] MMAs reading the stage have retired
-    uint64_t* accum_full = bars + 3 * Cfg::STAGES;          // accumulators of the current tile complete
-    uint64_t* tmem_empty = accum_full + 1;                  // epilogue has drained the accumulators
-    uint64_t* peer_full = tmem_empty + 1;                   // [STAGES] 2-CTA MMA, leader only: the PEER's TMA bytes of the stage landed
+    uint64_t* accum_full = bars + 3 * Cfg::STAGES;          // [ACC_BUFS] accumulators of the current tile complete
+    uint64_t* tmem_empty = accum_full + Cfg::ACC_BUFS;      // [ACC_BUFS] epilogue has drained the accumulators
+    uint64_t* peer_full = tmem_empty + Cfg::ACC_BUFS;       // [STAGES] 2-CTA MMA, leader only: the PEER's TMA bytes of the stage landed
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(peer_full + Cfg::STAGES);
     float* bias_s = reinterpret_cast<float*>(smem + (size_t)Cfg::STAGES * Cfg::STAGE_BYTES + 512);   // [N]
     float* stage_base = bias_s + Cfg::MAX_N;                // [4 warps][32][20]
@@ -108,9 +118,10 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
 
     auto a_hi = [&](int s) { return smem + (size_t)s * Cfg::STAGE_BYTES; };
     auto a_lo = [&](int s) { return smem + (size_t)s * Cfg::STAGE_BYTES + Cfg::A_BYTES; };
-    auto w_hi = [&](int s) { return smem + (size_t)s * Cfg::STAGE_BYTES + 2 * Cfg::A_BYTES; };
+    auto w_hi = [&](int s) { return smem + (size_t)s * Cfg::STAGE_BYTES + (kOne ? Cfg::A_BYTES + Cfg::A_BYTES / 2 : 2 * Cfg::A_BYTES); };
     auto w_lo = [&](int s) { return smem + (size_t)s * Cfg::STAGE_BYTES + 2 * Cfg::A_BYTES + Cfg::W_BYTES; };
     // kBf16: a_lo(s) holds bf16(A) [128x16] then bf16(A_lo); w_lo(s) holds bf16(W_hi) [BNx16] then bf16(W_lo)
+    // kOne: a_lo(s) holds bf16(A) [128x16], w_hi(s) the bf16 W tile [BNx16]
     auto a_b2 = [&](int s) { return a_lo(s) + Cfg::A_BYTES / 2; };
     auto w_b3 = [&](int s) { return w_lo(s) + Cfg::W_BYTES / 2; };
 
@@ -126,8 +137,10 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
             mbar_init(&empty[s], kCl == 2 ? 2 : 1);             // kCl = 2: the peer's TMA writes this stage too
             mbar_init(&peer_full[s], 1);
         }
-        mbar_init(accum_full, 1);
-        mbar_init(tmem_empty, kCl == 3 ? 2 * kTcEpiWarps : kTcEpiWarps);   // 2-CTA MMA: the leader waits for both epilogues
+        for (int b = 0; b < Cfg::ACC_BUFS; ++b) {
+            mbar_init(&accum_full[b], 1);
+            mbar_init(&tmem_empty[b], kCl == 3 ? 2 * kTcEpiWarps : kTcEpiWarps);   // 2-CTA MMA: the leader waits for both epilogues
+        }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -166,6 +179,12 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                     const int s = it % Cfg::STAGES;
                     if (kCl >= 2) mbar_wait_cluster(&empty[s], ((it / Cfg::STAGES) & 1) ^ 1);   // (arrivals come from the peer too)
                     else mbar_wait(&empty[s], ((it / Cfg::STAGES) & 1) ^ 1);
+                    if (kOne) {                                                // raw A + the bf16 W tile
+                        mbar_arrive_expect_tx(&full[s], Cfg::A_BYTES + Cfg::W_BYTES / 2);
+                        tma_load_2d(a_hi(s), &map_a, &full[s], (kb0 + kb) * kTcBK, m0);
+                        tma_load_2d(w_hi(s), &map_whi, &full[s], (kb0 + kb) * kTcBK, n0);
+                        continue;
+                    }
                     mbar_arrive_expect_tx(&full[s], Cfg::A_BYTES + 2 * Cfg::W_BYTES);      // own A + the whole W tile (both halves)
                     tma_load_2d(a_hi(s), &map_a, &full[s], (kb0 + kb) * kTcBK, m0);        // k past K arrives as zeros
                     if (kCl == 2) {
@@ -259,6 +278,28 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                         }
                     }
             }
+        } else if (kOne && lane == 0) {
+            // one bf16 MMA per k-block, into the accumulator buffer of the tile's parity
+            constexpr uint32_t idesc16 = umma_idesc_bf16(128, BN);
+            int it = 0, j = 0;
+            for (int tile = worker; tile < n_tiles; tile += n_workers, ++j) {
+                const int b = j & 1;
+                const uint32_t d_acc = tmem_base + (uint32_t)(b * BN);
+                if (j >= 2) {                                              // tile j-2's epilogue has drained buffer b
+                    mbar_wait(&tmem_empty[b], (uint32_t)((j >> 1) - 1) & 1u);
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                }
+                for (int kb = 0; kb < nkb; ++kb, ++it) {
+                    const int s = it % Cfg::STAGES;
+                    mbar_wait(&full[s], (it / Cfg::STAGES) & 1);           // W tile landed
+                    mbar_wait(&ready[s], (it / Cfg::STAGES) & 1);          // bf16(A) written
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    umma_bf16(d_acc, umma_desc_sw32(smem_u32(a_lo(s))), umma_desc_sw32(smem_u32(w_hi(s))), idesc16,
+                              kb > 0 ? 1u : 0u);
+                    umma_commit(&empty[s]);
+                }
+                umma_commit(&accum_full[b]);
+            }
         } else if (lane == 0) {
             constexpr uint32_t idesc = umma_idesc_tf32(128, BN);
             const uint32_t d_main = tmem_base, d_corr = tmem_base + (uint32_t)BN;
@@ -336,19 +377,22 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                 for (int i = 0; i < Cfg::A_BYTES / 16 / kTcTransformThreads; ++i) {
                     const int idx = t + i * kTcTransformThreads;
                     const float4 v = hi[idx];
-                    if (kBf16) {
+                    if (kBf16 || kOne) {
                         // source: fp32 tile, SWIZZLE_64B (16-byte chunk c of row r sits at chunk c ^ ((r >> 1) & 3));
-                        // destinations: two bf16 tiles, SWIZZLE_32B (rows of 32 bytes, chunk cd at cd ^ ((r >> 2) & 1))
+                        // destinations: bf16 tiles, SWIZZLE_32B (rows of 32 bytes, chunk cd at cd ^ ((r >> 2) & 1))
                         const int r = idx >> 2, c = (idx & 3) ^ ((r >> 1) & 3);          // logical columns 4c .. 4c+3
                         const uint32_t off = (uint32_t)(r * 32 + (((c >> 1) ^ ((r >> 2) & 1)) << 4) + ((c & 1) << 3));
                         __nv_bfloat162 p0 = __floats2bfloat162_rn(v.x, v.y), p1 = __floats2bfloat162_rn(v.z, v.w);
-                        __nv_bfloat162 q0 = __floats2bfloat162_rn(v.x - tf32_trunc(v.x), v.y - tf32_trunc(v.y));
-                        __nv_bfloat162 q1 = __floats2bfloat162_rn(v.z - tf32_trunc(v.z), v.w - tf32_trunc(v.w));
-                        uint2 full_v, lo_v;
+                        uint2 full_v;
                         full_v.x = *reinterpret_cast<uint32_t*>(&p0); full_v.y = *reinterpret_cast<uint32_t*>(&p1);
-                        lo_v.x = *reinterpret_cast<uint32_t*>(&q0); lo_v.y = *reinterpret_cast<uint32_t*>(&q1);
                         *reinterpret_cast<uint2*>(a_lo(s) + off) = full_v;                // bf16(A)
-                        *reinterpret_cast<uint2*>(a_b2(s) + off) = lo_v;                  // bf16(A - trunc_tf32(A))
+                        if (kBf16) {
+                            __nv_bfloat162 q0 = __floats2bfloat162_rn(v.x - tf32_trunc(v.x), v.y - tf32_trunc(v.y));
+                            __nv_bfloat162 q1 = __floats2bfloat162_rn(v.z - tf32_trunc(v.z), v.w - tf32_trunc(v.w));
+                            uint2 lo_v;
+                            lo_v.x = *reinterpret_cast<uint32_t*>(&q0); lo_v.y = *reinterpret_cast<uint32_t*>(&q1);
+                            *reinterpret_cast<uint2*>(a_b2(s) + off) = lo_v;              // bf16(A - trunc_tf32(A))
+                        }
                     } else {
                         float4 vl;
                         vl.x = to_tf32_rna(v.x - tf32_trunc(v.x)); vl.y = to_tf32_rna(v.y - tf32_trunc(v.y));
@@ -370,7 +414,7 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
         const int c_end = (kTcEpiWarps == 8 && ew < 4) ? (BN > 128 ? 128 : BN) : BN;
         const bool has_gb = gb.ptr != nullptr;
         float* stage = stage_base + ew * (32 * 20);
-        const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16);
+        const uint32_t tbase0 = tmem_base + ((uint32_t)(q * 32) << 16);
         int j = 0;
         for (int tile = worker; tile < n_tiles; tile += n_workers, ++j) {
             const int slice = tile / n_tiles_mn, t_mn = tile - slice * n_tiles_mn;
@@ -403,7 +447,9 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
 #ifdef DIGAT_TC_TIMING
             const long long e0 = clock64();
 #endif
-            mbar_wait(accum_full, (uint32_t)j & 1u);
+            const int b = Cfg::ACC_BUFS == 2 ? (j & 1) : 0;                // accumulator buffer of this tile
+            const uint32_t tbase = tbase0 + (uint32_t)(b * BN);
+            mbar_wait(&accum_full[b], (uint32_t)(Cfg::ACC_BUFS == 2 ? j >> 1 : j) & 1u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #ifdef DIGAT_TC_TIMING
             const long long e1 = clock64();
@@ -416,11 +462,12 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                     : "=r"(rm[0]), "=r"(rm[1]), "=r"(rm[2]), "=r"(rm[3]), "=r"(rm[4]), "=r"(rm[5]), "=r"(rm[6]), "=r"(rm[7]),
                       "=r"(rm[8]), "=r"(rm[9]), "=r"(rm[10]), "=r"(rm[11]), "=r"(rm[12]), "=r"(rm[13]), "=r"(rm[14]), "=r"(rm[15])
                     : "r"(tbase + (uint32_t)c));
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                    : "=r"(rc[0]), "=r"(rc[1]), "=r"(rc[2]), "=r"(rc[3]), "=r"(rc[4]), "=r"(rc[5]), "=r"(rc[6]), "=r"(rc[7]),
-                      "=r"(rc[8]), "=r"(rc[9]), "=r"(rc[10]), "=r"(rc[11]), "=r"(rc[12]), "=r"(rc[13]), "=r"(rc[14]), "=r"(rc[15])
-                    : "r"(tbase + (uint32_t)(BN + c)));
+                if (!kOne)                                                 // correction accumulator
+                    asm volatile(
+                        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                        : "=r"(rc[0]), "=r"(rc[1]), "=r"(rc[2]), "=r"(rc[3]), "=r"(rc[4]), "=r"(rc[5]), "=r"(rc[6]), "=r"(rc[7]),
+                          "=r"(rc[8]), "=r"(rc[9]), "=r"(rc[10]), "=r"(rc[11]), "=r"(rc[12]), "=r"(rc[13]), "=r"(rc[14]), "=r"(rc[15])
+                        : "r"(tbase + (uint32_t)(BN + c)));
 #pragma unroll
                 for (int v4 = 0; v4 < 4; ++v4) {
                     const int col = n0 + c + v4 * 4;
@@ -432,7 +479,7 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                 issue_group(c_begin);
             } else if (lane == 0) {
                 if (kCl == 3 && cl_rank == 1) mbar_arrive_cluster(tmem_empty, 0);
-                else mbar_arrive(tmem_empty);                          // nothing to drain for this warp (BN <= 128)
+                else mbar_arrive(&tmem_empty[b]);                      // nothing to drain for this warp (BN <= 128)
             }
 #pragma unroll 1
             for (int c = c_begin; c < c_end; c += 16) {
@@ -440,7 +487,8 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                 float o[16];
 #pragma unroll
                 for (int i = 0; i < 16; ++i)
-                    o[i] = (__uint_as_float(rm[i]) + __uint_as_float(rc[i])) + ((n0 + c + i < N && slice == 0) ? bias_s[n0 + c + i] : 0.f);
+                    o[i] = (kOne ? __uint_as_float(rm[i]) : __uint_as_float(rm[i]) + __uint_as_float(rc[i])) +
+                           ((n0 + c + i < N && slice == 0) ? bias_s[n0 + c + i] : 0.f);
 #pragma unroll
                 for (int v4 = 0; v4 < 4; ++v4) {
                     float4 gv = gq[v4];
@@ -456,7 +504,7 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
                     __syncwarp();
                     if (lane == 0) {
                         if (kCl == 3 && cl_rank == 1) mbar_arrive_cluster(tmem_empty, 0);   // the leader issues the next tile's MMAs
-                        else mbar_arrive(tmem_empty);
+                        else mbar_arrive(&tmem_empty[b]);
                     }
                 }
                 __syncwarp();
@@ -501,17 +549,17 @@ gemm_tf32x3_persistent_kernel(const __grid_constant__ CUtensorMap map_a, const _
 static int g_tc_cluster = 0;   // 0 = independent CTAs, 1 = W multicast across CTA pairs, 2 = 2-CTA MMA (digat_debug_set_gemm_variant 6 / 7 / 8)
 
 // Launch of one persistent instantiation; kCl = 2 goes through cudaLaunchKernelEx with a (2,1,1) cluster.
-template <int BN, bool kBf16, int kCl>
+template <int BN, bool kBf16, int kCl, bool kOne = false>
 int launch_tf32x3_persistent_inst(const CUtensorMap& ma, const CUtensorMap& mh, const CUtensorMap& ml, const CUtensorMap& m3,
                                   const float* bias, float* C, int ldc, int M, int N, int K, GroupBias gb, int units, int sm_count,
                                   cudaStream_t st) {
-    using Cfg = TcPersistCfg<BN, kCl>;
-    auto kernel = gemm_tf32x3_persistent_kernel<BN, kBf16, kCl>;
+    using Cfg = TcPersistCfg<BN, kCl, kOne>;
+    auto kernel = gemm_tf32x3_persistent_kernel<BN, kBf16, kCl, kOne>;
     if (int rc_ = ensure_dynamic_smem(kernel, (size_t)Cfg::SMEM)) return rc_;
     if (kCl == 1) {
         const int grid = units < sm_count ? units : sm_count;
         kernel<<<grid, kTcPersistThreads, Cfg::SMEM, st>>>(ma, mh, ml, m3, bias, C, ldc, M, N, K, gb);
-        return check_launch("digat_linear_tf32x3(persistent)");
+        return check_launch(kOne ? "digat_linear_bf16" : "digat_linear_tf32x3(persistent)");
     }
     cudaLaunchConfig_t cfg{};
     cfg.blockDim = dim3(kTcPersistThreads);

@@ -83,12 +83,18 @@ def _ends_tensor(sizes, device):
 
 class PackedWeight:
     """A projection weight in kernel layout: fp32 [N,K] (nn.Linear layout) plus, when the tcgen05 GEMM can take it
-    (N % 16 == 0, K % 4 == 0), its two TF32 planes hi = rna_tf32(W), lo = rna_tf32(W - hi) (digat_split_tf32)."""
-    __slots__ = ('w', 'hi', 'lo', 'hb', 'lb')
+    (N % 16 == 0, K % 4 == 0), its two TF32 planes hi = rna_tf32(W), lo = rna_tf32(W - hi) (digat_split_tf32).
+    bf16=True adds wb = bf16_rn(W): linear() then runs this weight's products on the BF16 GEMM (digat_linear_bf16)."""
+    __slots__ = ('w', 'hi', 'lo', 'hb', 'lb', 'wb')
 
-    def __init__(self, w):
+    def __init__(self, w, bf16=False):
         self.w = w.detach().float().contiguous()
-        self.hi = self.lo = self.hb = self.lb = None
+        self.hi = self.lo = self.hb = self.lb = self.wb = None
+        if bf16:
+            if self.w.shape[0] % 16 != 0 or self.w.shape[0] > 1280 or self.w.shape[1] % 8 != 0:
+                raise RuntimeError('PackedWeight: the BF16 GEMM needs N %% 16 == 0, N <= 1280, K %% 8 == 0 (got %s)'
+                                   % (tuple(self.w.shape),))
+            self.wb = self.w.to(torch.bfloat16)             # round to nearest even
         if self.w.shape[0] % 16 == 0 and self.w.shape[1] % 4 == 0:
             self.hi, self.lo = torch.empty_like(self.w), torch.empty_like(self.w)
             _lib.call('digat_split_tf32', self.w.data_ptr(), self.hi.data_ptr(), self.lo.data_ptr(), self.w.numel(),
@@ -121,6 +127,9 @@ def linear(A, W, bias=None, relu=False, M=None, K=None, lda=None, out=None, grou
     c_rows [M] int32 ascending (tensor-core path only, ``out`` required): product row m lands in out[c_rows[m]] and takes
     the group bias of that row; the other rows of ``out`` are left untouched."""
     w = W.w if isinstance(W, PackedWeight) else W
+    bf16 = isinstance(W, PackedWeight) and W.wb is not None
+    if bf16 and relu:
+        raise RuntimeError('linear: the BF16 GEMM has no relu epilogue')
     N = w.shape[0]
     if K is None:
         K = w.shape[1]
@@ -137,7 +146,10 @@ def linear(A, W, bias=None, relu=False, M=None, K=None, lda=None, out=None, grou
     m_dense = out.shape[0] if c_rows is not None else M
     bf16c = GEMM_BF16_CORRECTIONS and isinstance(W, PackedWeight) and W.hb is not None and m_dense >= BF16C_MIN_ROWS and \
         (K & 7) == 0 and not relu
-    if c_rows is not None:
+    if bf16:                                                            # every M, with or without c_rows
+        _lib.call('digat_linear_bf16', A.data_ptr(), lda, W.wb.data_ptr(), W.wb.stride(0), _ptr(bias), out.data_ptr(),
+                  out.stride(0), M, N, K, _ptr(group_bias), group_rows, group_col0, gcols, gld, _ptr(c_rows), _stream())
+    elif c_rows is not None:
         if not (isinstance(W, PackedWeight) and W.hi is not None) or relu:
             raise RuntimeError('linear: c_rows needs a PackedWeight with TF32 planes and no relu')
         if bf16c:
@@ -307,13 +319,23 @@ class DIGAT(GraphEncoder):
         self.userAttention.initialize()
 
     # ---------------------------------------------------------------------------------- packed weights
+    def _bf16_projections(self):
+        """True when projection_precision selects the BF16 node projections; raises on an unknown value."""
+        mode = self.projection_precision
+        if mode not in ('fp32', 'bf16'):
+            raise ValueError("projection_precision must be 'fp32' or 'bf16', got %r" % (mode,))
+        return mode == 'bf16'
+
     def _weights(self):
-        """Kernel-side weight layout, rebuilt only when a parameter changed (optimizer step / load_state_dict):
+        """Kernel-side weight layout, rebuilt only when a parameter changed (optimizer step / load_state_dict) or
+        projection_precision did:
         * per layer and graph: [W; ffn1; ffn2] stacked to [3D, D] so h, K1, K2 come out of ONE projection GEMM;
         * attention K matrices transposed, so the folded query v = K^T (Q q + b) is a plain linear;
-        * [user_news_Q; userAttention.Q] stacked: both queries of the user context come from one GEMM on c_n."""
+        * [user_news_Q; userAttention.Q] stacked: both queries of the user context come from one GEMM on c_n;
+        * projection_precision = 'bf16': Wcat and featureAffine also carry their bf16 plane (PackedWeight.wb)."""
+        bf16 = self._bf16_projections()
         params = list(self.parameters())
-        key = tuple((p.data_ptr(), p._version) for p in params)
+        key = tuple((p.data_ptr(), p._version) for p in params) + (bf16,)
         if self._packed is not None and key == self._packed_key:
             return self._packed
         dev = params[0].device
@@ -330,7 +352,8 @@ class DIGAT(GraphEncoder):
                     f2 = getattr(self, g + '_graph_attention_ffn2')[i]
                     f3 = getattr(self, g + '_graph_attention_ffn3')[i]
                     av = getattr(self, g + '_graph_attention_a')[i]
-                    w[g, i, 'Wcat'] = PackedWeight(torch.cat([W.weight, f1.weight, f2.weight], 0).float().contiguous())
+                    w[g, i, 'Wcat'] = PackedWeight(torch.cat([W.weight, f1.weight, f2.weight], 0).float().contiguous(),
+                                                   bf16=bf16)
                     w[g, i, 'bcat'] = torch.cat([W.bias, torch.zeros(2 * D, device=dev)], 0).float().contiguous()
                     w[g, i, 'W3'] = PackedWeight(f3.weight.detach().float().contiguous())
                     w[g, i, 'b3'] = f3.bias.detach().float().contiguous()
@@ -356,7 +379,7 @@ class DIGAT(GraphEncoder):
                     bs.append(f3.bias.detach().float())
                 w['uctx_W', j] = PackedWeight(torch.cat(Ws, 0).contiguous())
                 w['uctx_b', j] = torch.cat(bs, 0).contiguous()
-            w['fa_W'] = PackedWeight(self.featureAffine.weight.detach().float().contiguous())
+            w['fa_W'] = PackedWeight(self.featureAffine.weight.detach().float().contiguous(), bf16=bf16)
             w['fa_b'] = self.featureAffine.bias.detach().float().contiguous()
             w['topic'] = self.topic_node_embedding.detach().float().contiguous()
         self._packed, self._packed_key = w, key
@@ -438,6 +461,10 @@ class DIGAT(GraphEncoder):
         return graph_layer_fwd(P, w[g, i, 'a'], adj, X, adj_index=adj_index, csr=csr), None
 
     prune_user_nodes = True      # inference only; switch off to evaluate every node of every user graph
+    # Arithmetic of the node projections at inference (the per-layer h | K1 | K2 GEMM of both graphs and featureAffine):
+    # 'fp32' (3xTF32, fp32-level accuracy) or 'bf16' (operands rounded to bf16, fp32 accumulation; DESIGN.md section 4.8).
+    # Every other GEMM, and the training path (autograd_ops.encode_with_grad), stays fp32 in either mode.
+    projection_precision = 'fp32'
     precompute_user_csr = True   # user-graph CSR records built once per batch (build_graph_csr) instead of in every layer launch
 
     def _user_csr(self, Au, prune, share, first_rows):

@@ -91,6 +91,14 @@ int digat_linear_tf32_bf16c(const float* A, int lda, const float* W_hi, const vo
                             const float* group_bias, int group_rows, int group_col0, int group_cols, int group_ld,
                             const int32_t* c_row_index, void* stream);
 
+/* C = bf16_rn(A) * W_b^T (+bias)(+row-group bias), fp32 accumulation.  W_b = bf16_rn(W) [N,K] (row pitch ldw).
+ * Same bias / group-bias / c_row_index semantics and alignment rules as digat_linear_tf32x3; K, ldw % 8 == 0, N <= 1280.
+ * One tcgen05 kind::f16 MMA per 16-wide k-block; every M takes the same kernel, and an output row depends on its A row
+ * and W only.  The opt-in inference precision of the DIGAT node projections (DIGAT.projection_precision = 'bf16'). */
+int digat_linear_bf16(const float* A, int lda, const void* W_b, int ldw, const float* bias, float* C, int ldc,
+                      int M, int N, int K, const float* group_bias, int group_rows, int group_col0, int group_cols,
+                      int group_ld, const int32_t* c_row_index, void* stream);
+
 /* Split-K form of digat_linear_tf32x3 (no bias): the contraction range [0,K) is cut into kbatches equal slices and slice
  * s writes its partial product to C + s * c_batch_stride (elements); the caller sums the slabs (digat_colsum over a
  * [kbatches, M*ldc] view: exact fp32 adds in slice order).  Used for weight gradients dW = dC^T A, whose contraction
