@@ -18,14 +18,10 @@ SIGNATURES = {
     'digat_split_tf32': [c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
     'digat_linear_tf32x3': [c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                             c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
-    'digat_split_bf16': [c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
-    'digat_linear_tf32_bf16c': [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
-                                c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     'digat_linear_bf16': [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                           c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     'digat_linear_tf32x3_splitk': [c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                    c_int64, c_void_p],
-    'digat_debug_set_gemm_variant': [c_int],
     'digat_debug_set_layer_mode': [c_int],
     'digat_graph_layer_fwd': [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                               c_void_p, ctypes.c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
@@ -127,7 +123,7 @@ def require_device(device_index: int):
     _device_ok[device_index] = True
 
 
-_NON_KERNEL = ('digat_graph_layer_supports_row_active', 'digat_graph_layer_csr_training_supported', 'digat_graph_layer_bwd_csr_parts', 'digat_abi_version', 'digat_device_check', 'digat_debug_set_gemm_variant', 'digat_debug_set_layer_mode',
+_NON_KERNEL = ('digat_graph_layer_supports_row_active', 'digat_graph_layer_csr_training_supported', 'digat_graph_layer_bwd_csr_parts', 'digat_abi_version', 'digat_device_check', 'digat_debug_set_layer_mode',
                'digat_reduce_workspace_floats')
 _launches = 0
 _profile = None      # list of (name, args, start_event, end_event) while bench.py's per-kernel pass is running

@@ -4,7 +4,6 @@
 #include "gemm_simt.cuh"
 #include "gemm_small.cuh"
 #include "gemm_tcgen05.cuh"
-#include "gemm_tcgen05_pair.cuh"
 #include "gemm_tcgen05_persistent.cuh"
 #include "gemm_bf16.cuh"
 #include "pair_attention.cuh"
@@ -80,34 +79,6 @@ int digat_linear_tf32x3_splitk(const float* A, int lda, const float* W_hi, const
     return launch_linear_tf32x3(A, lda, W_hi, W_lo, ldw, nullptr, C, ldc, M, N, K, gb, as_stream(stream));
 }
 
-int digat_split_bf16(const float* W, void* W_hb, void* W_lb, int64_t count, void* stream) {
-    DIGAT_REQUIRE(W && W_hb && W_lb, "digat_split_bf16: null pointer");
-    if (count <= 0) return DIGAT_OK;
-    split_bf16_kernel<<<(unsigned)((count + 255) / 256), 256, 0, as_stream(stream)>>>(
-        W, reinterpret_cast<__nv_bfloat16*>(W_hb), reinterpret_cast<__nv_bfloat16*>(W_lb), count);
-    return check_launch("digat_split_bf16");
-}
-
-int digat_linear_tf32_bf16c(const float* A, int lda, const float* W_hi, const void* W_hb, const void* W_lb, int ldw,
-                            const float* bias, float* C, int ldc, int M, int N, int K, const float* group_bias,
-                            int group_rows, int group_col0, int group_cols, int group_ld, const int32_t* c_row_index,
-                            void* stream) {
-    if (M == 0) return DIGAT_OK;
-    DIGAT_REQUIRE(A && W_hi && W_hb && W_lb && C, "digat_linear_tf32_bf16c: null pointer");
-    DIGAT_REQUIRE(M > 0 && N > 0 && K > 0 && (K & 7) == 0 && (lda & 3) == 0 && (ldw & 7) == 0 && (ldc & 3) == 0 &&
-                  lda >= K && ldw >= K && ldc >= N && N % 16 == 0 && N <= 1280,
-                  "digat_linear_tf32_bf16c: needs K, ldw multiples of 8, lda, ldc multiples of 4, N a multiple of 16 and <= 1280");
-    DIGAT_REQUIRE(aligned16(A) && aligned16(W_hi) && aligned16(W_hb) && aligned16(W_lb) && aligned16(C) &&
-                  (!bias || aligned16(bias)), "digat_linear_tf32_bf16c: pointers must be 16-byte aligned");
-    GroupBias gb{group_bias, group_rows, group_col0, group_cols, group_ld, c_row_index};
-    DIGAT_REQUIRE(gb.ptr == nullptr || (gb.rows > 0 && gb.col0 >= 0 && gb.cols > 0 && gb.col0 + gb.cols <= N &&
-                                        (gb.col0 & 3) == 0 && (gb.cols & 3) == 0 && (gb.ld & 3) == 0 && gb.ld >= gb.cols &&
-                                        aligned16(gb.ptr)), "digat_linear_tf32_bf16c: bad row-group bias");
-    if (N % 240 == 0)
-        return launch_tf32x3_persistent<240>(A, lda, W_hi, nullptr, ldw, bias, C, ldc, M, N, K, gb, as_stream(stream), W_hb, W_lb);
-    return launch_tf32x3_persistent<208>(A, lda, W_hi, nullptr, ldw, bias, C, ldc, M, N, K, gb, as_stream(stream), W_hb, W_lb);
-}
-
 int digat_linear_bf16(const float* A, int lda, const void* W_b, int ldw, const float* bias, float* C, int ldc,
                       int M, int N, int K, const float* group_bias, int group_rows, int group_col0, int group_cols,
                       int group_ld, const int32_t* c_row_index, void* stream) {
@@ -118,19 +89,6 @@ int digat_linear_bf16(const float* A, int lda, const void* W_b, int ldw, const f
 
 int digat_debug_set_layer_mode(int mode) {
     g_layer_mode = mode;
-    return DIGAT_OK;
-}
-
-int digat_debug_set_gemm_variant(int variant) {
-    if (variant >= 6 && variant <= 8) {          // persistent kernel: 6 = independent CTAs, 7 = W multicast, 8 = 2-CTA MMA
-        g_tc_cluster = variant - 6;
-        return DIGAT_OK;
-    }
-    if (variant >= 10 && variant <= 13) {        // tile width of the few-hundred-row GEMMs: 128 (off), 64, 32, 16
-        g_tc_small_bn = 128 >> (variant - 10);
-        return DIGAT_OK;
-    }
-    g_tc_variant = variant;
     return DIGAT_OK;
 }
 

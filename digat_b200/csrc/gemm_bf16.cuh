@@ -2,7 +2,7 @@
 //
 //   C[M,N] = bf16_rn(A) * W_b^T (+ bias) (+ row-group bias),   W_b = bf16_rn(W) [N,K], fp32 accumulation in TMEM
 //
-// It runs the persistent kernel of gemm_tcgen05_persistent.cuh with kOne = true, for every M: the raw fp32 A tile lands
+// It runs the persistent kernel of gemm_tcgen05_persistent.cuh with kBf16 = true, for every M: the raw fp32 A tile lands
 // by TMA exactly as for 3xTF32 (16-wide k-blocks, SWIZZLE_64B), the transform warps round it to a bf16 SWIZZLE_32B
 // tile, W arrives as one bf16 plane, and each k-block is ONE tcgen05.mma.kind::f16 (K = 16) into one accumulator.  With
 // one accumulator per tile two of them fit in TMEM (2 x 240 or 2 x 208 columns), so the epilogue of tile t overlaps the
@@ -23,8 +23,7 @@ int launch_bf16_persistent(const float* A, int lda, const void* W_b, int ldw, co
     int rc;
     if ((rc = make_tensor_map_2d(&ma, A, M, K, lda, 128, kTcBK, CU_TENSOR_MAP_SWIZZLE_64B)) != DIGAT_OK) return rc;
     if ((rc = make_tensor_map_2d_bf16(&mw, W_b, N, K, ldw, BN, kTcBK, CU_TENSOR_MAP_SWIZZLE_32B)) != DIGAT_OK) return rc;
-    const int units = ((N + BN - 1) / BN) * ((M + 127) / 128);
-    return launch_tf32x3_persistent_inst<BN, false, 1, true>(ma, mw, mw, mw, bias, C, ldc, M, N, K, gb, units, di->sm_count, st);
+    return launch_persistent_inst<BN, true>(ma, mw, mw, bias, C, ldc, M, N, K, gb, di->sm_count, st);
 }
 
 inline int launch_linear_bf16(const float* A, int lda, const void* W_b, int ldw, const float* bias, float* C, int ldc,
@@ -37,10 +36,7 @@ inline int launch_linear_bf16(const float* A, int lda, const void* W_b, int ldw,
                   "(M=%d N=%d K=%d lda=%d ldw=%d ldc=%d)", M, N, K, lda, ldw, ldc);
     DIGAT_REQUIRE(aligned16(A) && aligned16(W_b) && aligned16(C) && (!bias || aligned16(bias)),
                   "digat_linear_bf16: pointers must be 16-byte aligned");
-    DIGAT_REQUIRE(gb.ptr == nullptr || (gb.rows > 0 && gb.col0 >= 0 && gb.cols > 0 && gb.col0 + gb.cols <= N &&
-                                        (gb.col0 & 3) == 0 && (gb.cols & 3) == 0 && (gb.ld & 3) == 0 && gb.ld >= gb.cols &&
-                                        aligned16(gb.ptr)),
-                  "digat_linear_bf16: bad row-group bias (col0/cols must be multiples of 4)");
+    if (int rc_ = check_group_bias("digat_linear_bf16", gb, N)) return rc_;
     if (N % 240 == 0) return launch_bf16_persistent<240>(A, lda, W_b, ldw, bias, C, ldc, M, N, K, gb, st);
     return launch_bf16_persistent<208>(A, lda, W_b, ldw, bias, C, ldc, M, N, K, gb, st);
 }

@@ -7,17 +7,16 @@
 // This is the projection GEMM of the DIGAT layer: h | K1 | K2 = X * [W; ffn1; ffn2]^T (reference
 // graphEncoders.py:146-148 / 166-168), M = batch*nodes, N = 3D = 1200, K = D = 400.
 //
-// CTA = 192 threads, one output tile of (MH*128) x BN:
+// CTA = 192 threads, one output tile of 128 x BN:
 //   warp 0      TMA producer: per k-block (16 fp32 = one 64-byte swizzle row) loads the raw A tile and both W planes
 //   warps 2..5  operand transform: split the raw fp32 A tile in smem into A_hi (in place) and A_lo, fence to the
 //               async proxy, signal the MMA warp; after the main loop the same warps run the epilogue
 //               (tcgen05.ld TMEM -> registers, + bias, 128-bit global stores)
-//   warp 1      MMA issuer (one elected lane): 3 x tcgen05.mma.kind::tf32 per 8-wide k-step and 128-row half, commit
-//               to the stage's "empty" barrier; owns the TMEM allocation (MH*BN fp32 columns).
+//   warp 1      MMA issuer (one elected lane): 3 x tcgen05.mma.kind::tf32 per 8-wide k-step, commit to the stage's
+//               "empty" barrier; owns the TMEM allocation (2*BN fp32 columns).
 // Pipeline: full[s] (TMA bytes landed) -> ready[s] (A split done) -> MMA -> empty[s] (tcgen05.commit) -> TMA.
 #pragma once
 #include "common.cuh"
-#include <cuda_bf16.h>
 #include "tma.cuh"
 #include "gemm_simt.cuh"   // GroupBias
 
@@ -27,6 +26,8 @@ constexpr int kTcBK = 16;                       // fp32 elements per k-block = 6
 constexpr int kTcThreads = 192;
 constexpr int kTcTransformThreads = 128;
 constexpr int kTcPrefetchBlocks = 40;          // M blocks between a CTA and the block whose A rows it prefetches into L2
+constexpr int kTcSmallRows = 1024;             // GEMMs of at most this many rows take 32-wide tiles
+constexpr int kTcBigRows = 16384;              // GEMMs of more rows take the persistent kernel or the wide tiles
 
 // K-major operand tile, SWIZZLE_64B: rows of 64 bytes, 8-row groups of 512 bytes (SBO), version 1 (sm_100).
 __device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr) {
@@ -86,12 +87,12 @@ __device__ __forceinline__ float to_tf32_rna(float x) {
     return __uint_as_float(r);
 }
 
-// SPLIT: the correction products (A_lo*W_hi + A_hi*W_lo, ~2^-11 of the main term) get their own TMEM accumulator.
+// The correction products (A_lo*W_hi + A_hi*W_lo, ~2^-11 of the main term) get their own TMEM accumulator.
 // The tensor core adds into the fp32 accumulator with truncation, aligned to the accumulator's exponent; keeping the
 // small terms out of the large accumulator removes most of that error (measured: see profiles/ and DESIGN.md).
-template <int BN, int MH, bool SPLIT>
+template <int BN>
 struct TcCfg {
-    static constexpr int BM = 128 * MH;
+    static constexpr int BM = 128;
     static constexpr int A_BYTES = BM * kTcBK * 4;             // one plane of the A tile
     static constexpr int W_BYTES = BN * kTcBK * 4;
     static constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * W_BYTES;
@@ -99,7 +100,7 @@ struct TcCfg {
     // epilogue overlaps the other's main loop.  The other widths own the SM (up to 512 TMEM columns, ~200 KB).
     static constexpr int SMEM_BUDGET = (BN == 128 ? 108 : 200) * 1024;
     static constexpr int STAGES = SMEM_BUDGET / STAGE_BYTES > 6 ? 6 : SMEM_BUDGET / STAGE_BYTES;
-    static constexpr int ACC_COLS = MH * BN * (SPLIT ? 2 : 1);
+    static constexpr int ACC_COLS = 2 * BN;                    // main + correction accumulators
     static constexpr int TMEM_COLS = (ACC_COLS <= 32) ? 32 : (ACC_COLS <= 64) ? 64 : (ACC_COLS <= 128) ? 128
                                      : (ACC_COLS <= 256) ? 256 : 512;
     static constexpr size_t SMEM = (size_t)STAGES * STAGE_BYTES + 1024 /*alignment slack*/ + 256 /*barriers*/;
@@ -109,12 +110,12 @@ struct TcCfg {
     static_assert(STAGES >= 2, "not enough shared memory for a pipeline");
 };
 
-template <int BN, int MH, bool SPLIT>
+template <int BN>
 __global__ void __launch_bounds__(kTcThreads, BN == 128 ? 2 : 1)
 gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_whi,
                    const __grid_constant__ CUtensorMap map_wlo, const float* __restrict__ bias,
                    float* __restrict__ C, int ldc, int M, int N, int K, GroupBias gb) {
-    using Cfg = TcCfg<BN, MH, SPLIT>;
+    using Cfg = TcCfg<BN>;
     extern __shared__ __align__(1024) uint8_t smem_raw[];   // SWIZZLE_64B operand tiles: keep 1024-byte alignment
     uint8_t* smem = smem_raw;                               // stays a __shared__ pointer (LDS/STS in the transform warps)
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)Cfg::STAGES * Cfg::STAGE_BYTES);
@@ -156,9 +157,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-#ifdef DIGAT_TC_TIMING
-    const long long t_start = clock64();
-#endif
 
     if (warp == 0) {
         // ------------------------------------------------------------------ TMA producer
@@ -196,18 +194,14 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
                 mbar_wait(&full[s], (kb / Cfg::STAGES) & 1);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint64_t d_whi = umma_desc_sw64(smem_u32(w_hi(s))), d_wlo = umma_desc_sw64(smem_u32(w_lo(s)));
+                const uint64_t d_ahi = umma_desc_sw64(smem_u32(a_hi(s)));
+                const uint32_t d_main = tmem_base, d_corr = tmem_base + (uint32_t)BN;
 #pragma unroll
-                for (int h = 0; h < MH; ++h) {
-                    const uint64_t d_ahi = umma_desc_sw64(smem_u32(a_hi(s) + h * 128 * kTcBK * 4));
-                    const uint32_t d_main = tmem_base + (uint32_t)(h * BN);
-                    const uint32_t d_corr = SPLIT ? tmem_base + (uint32_t)((MH + h) * BN) : d_main;
-#pragma unroll
-                    for (int k = 0; k < kTcBK / 8; ++k) {
-                        const uint64_t koff = (uint64_t)((k * 8 * 4) >> 4);   // 32 bytes per k-step, in 16-byte units
-                        const uint32_t first = (kb > 0 || k > 0) ? 1u : 0u;
-                        umma_tf32(d_main, d_ahi + koff, d_whi + koff, idesc, first);
-                        umma_tf32(d_corr, d_ahi + koff, d_wlo + koff, idesc, SPLIT ? first : 1u);
-                    }
+                for (int k = 0; k < kTcBK / 8; ++k) {
+                    const uint64_t koff = (uint64_t)((k * 8 * 4) >> 4);   // 32 bytes per k-step, in 16-byte units
+                    const uint32_t first = (kb > 0 || k > 0) ? 1u : 0u;
+                    umma_tf32(d_main, d_ahi + koff, d_whi + koff, idesc, first);
+                    umma_tf32(d_corr, d_ahi + koff, d_wlo + koff, idesc, first);
                 }
             };
             auto issue_lo = [&](int kb) {                         // A_lo * W_hi, then release the stage
@@ -215,35 +209,21 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
                 mbar_wait(&ready[s], (kb / Cfg::STAGES) & 1);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint64_t d_whi = umma_desc_sw64(smem_u32(w_hi(s)));
+                const uint64_t d_alo = umma_desc_sw64(smem_u32(a_lo(s)));
+                const uint32_t d_corr = tmem_base + (uint32_t)BN;
 #pragma unroll
-                for (int h = 0; h < MH; ++h) {
-                    const uint64_t d_alo = umma_desc_sw64(smem_u32(a_lo(s) + h * 128 * kTcBK * 4));
-                    const uint32_t d_corr = SPLIT ? tmem_base + (uint32_t)((MH + h) * BN) : tmem_base + (uint32_t)(h * BN);
-#pragma unroll
-                    for (int k = 0; k < kTcBK / 8; ++k) {
-                        const uint64_t koff = (uint64_t)((k * 8 * 4) >> 4);
-                        umma_tf32(d_corr, d_alo + koff, d_whi + koff, idesc, 1u);
-                    }
+                for (int k = 0; k < kTcBK / 8; ++k) {
+                    const uint64_t koff = (uint64_t)((k * 8 * 4) >> 4);
+                    umma_tf32(d_corr, d_alo + koff, d_whi + koff, idesc, 1u);
                 }
                 umma_commit(&empty[s]);            // frees the smem stage once every MMA issued so far has retired
             };
             issue_raw(0);
-#ifdef DIGAT_TC_TIMING
-            const long long t_first = clock64();
-#endif
             for (int kb = 0; kb < nkb; ++kb) {
                 if (kb + 1 < nkb) issue_raw(kb + 1);
                 issue_lo(kb);
             }
             umma_commit(accum_full);               // accumulators complete
-#ifdef DIGAT_TC_TIMING
-            const long long t_issued = clock64();
-            mbar_wait(accum_full, 0);
-            const long long t_done = clock64();
-            if (blockIdx.x == 2 && ((blockIdx.y % 997) == 5 || (gridDim.y < 6 && blockIdx.y == 1)))
-                printf("tile(%d,%d): first MMA issued +%lld, all issued +%lld, accum done +%lld\n", blockIdx.x, blockIdx.y,
-                       t_first - t_start, t_issued - t_start, t_done - t_start);
-#endif
         }
     } else {
         // ------------------------------------------------------------------ operand transform, then epilogue
@@ -275,76 +255,64 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
         const int q = warp & 3;
         const bool has_gb = gb.ptr != nullptr;
         float* stage = reinterpret_cast<float*>(smem) + q * (32 * 20);     // per-warp 32 x (16+4) staging block
+        const int m = m0 + q * 32 + lane;
+        const bool row_ok = m < M;
+        const float* grow = (has_gb && row_ok) ? gb.ptr + (size_t)(m / gb.rows) * gb.ld - gb.col0 + n0 : nullptr;
+        const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16);
+        uint32_t rm[16], rc[16];
+        float4 gq[4];
+        auto issue_group = [&](int c) {
+            asm volatile(
+                "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                : "=r"(rm[0]), "=r"(rm[1]), "=r"(rm[2]), "=r"(rm[3]), "=r"(rm[4]), "=r"(rm[5]), "=r"(rm[6]), "=r"(rm[7]),
+                  "=r"(rm[8]), "=r"(rm[9]), "=r"(rm[10]), "=r"(rm[11]), "=r"(rm[12]), "=r"(rm[13]), "=r"(rm[14]), "=r"(rm[15])
+                : "r"(tbase + (uint32_t)c));
+            asm volatile(
+                "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                : "=r"(rc[0]), "=r"(rc[1]), "=r"(rc[2]), "=r"(rc[3]), "=r"(rc[4]), "=r"(rc[5]), "=r"(rc[6]), "=r"(rc[7]),
+                  "=r"(rc[8]), "=r"(rc[9]), "=r"(rc[10]), "=r"(rc[11]), "=r"(rc[12]), "=r"(rc[13]), "=r"(rc[14]), "=r"(rc[15])
+                : "r"(tbase + (uint32_t)(BN + c)));
 #pragma unroll
-        for (int h = 0; h < MH; ++h) {
-            const int m = m0 + h * 128 + q * 32 + lane;
-            const bool row_ok = m < M;
-            const float* grow = (has_gb && row_ok) ? gb.ptr + (size_t)(m / gb.rows) * gb.ld - gb.col0 + n0 : nullptr;
-            const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * BN);
-            uint32_t rm[16], rc[16];
-            float4 gq[4];
-            auto issue_group = [&](int c) {
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                    : "=r"(rm[0]), "=r"(rm[1]), "=r"(rm[2]), "=r"(rm[3]), "=r"(rm[4]), "=r"(rm[5]), "=r"(rm[6]), "=r"(rm[7]),
-                      "=r"(rm[8]), "=r"(rm[9]), "=r"(rm[10]), "=r"(rm[11]), "=r"(rm[12]), "=r"(rm[13]), "=r"(rm[14]), "=r"(rm[15])
-                    : "r"(tbase + (uint32_t)c));
-                if (SPLIT) {
-                    asm volatile(
-                        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                        : "=r"(rc[0]), "=r"(rc[1]), "=r"(rc[2]), "=r"(rc[3]), "=r"(rc[4]), "=r"(rc[5]), "=r"(rc[6]), "=r"(rc[7]),
-                          "=r"(rc[8]), "=r"(rc[9]), "=r"(rc[10]), "=r"(rc[11]), "=r"(rc[12]), "=r"(rc[13]), "=r"(rc[14]), "=r"(rc[15])
-                        : "r"(tbase + (uint32_t)(MH * BN + c)));
-                }
-#pragma unroll
-                for (int v4 = 0; v4 < 4; ++v4) {
-                    const int col = n0 + c + v4 * 4;       // col0 / cols are multiples of 4: a quad is entirely in or out
-                    gq[v4] = (grow != nullptr && col >= gb.col0 && col < gb.col0 + gb.cols)
-                                 ? *reinterpret_cast<const float4*>(grow + c + v4 * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            };
-            issue_group(0);
+            for (int v4 = 0; v4 < 4; ++v4) {
+                const int col = n0 + c + v4 * 4;       // col0 / cols are multiples of 4: a quad is entirely in or out
+                gq[v4] = (grow != nullptr && col >= gb.col0 && col < gb.col0 + gb.cols)
+                             ? *reinterpret_cast<const float4*>(grow + c + v4 * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        };
+        issue_group(0);
 #pragma unroll 1
-            for (int c = 0; c < BN; c += 16) {
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                float o[16];
+        for (int c = 0; c < BN; c += 16) {
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            float o[16];
 #pragma unroll
-                for (int i = 0; i < 16; ++i) {
-                    float v = __uint_as_float(rm[i]);
-                    if (SPLIT) v += __uint_as_float(rc[i]);          // main + correction accumulators (IEEE add)
-                    o[i] = v + bias_s[c + i];
-                }
+            for (int i = 0; i < 16; ++i)        // main + correction accumulators (IEEE add), then the bias
+                o[i] = (__uint_as_float(rm[i]) + __uint_as_float(rc[i])) + bias_s[c + i];
 #pragma unroll
-                for (int v4 = 0; v4 < 4; ++v4) {
-                    o[v4 * 4 + 0] += gq[v4].x; o[v4 * 4 + 1] += gq[v4].y;
-                    o[v4 * 4 + 2] += gq[v4].z; o[v4 * 4 + 3] += gq[v4].w;
-                }
-                if (c + 16 < BN) issue_group(c + 16);                // next group's loads overlap these stores
-                // A thread owns one ROW of the tile, so direct stores would scatter 16-byte pieces over 32 rows per
-                // instruction (measured: the epilogue was LSU-transaction-bound, 10.5k of 36k cycles per tile).  Stage the
-                // 32 x 16 block through shared memory (the pipeline stages are idle now) and write 64-byte row segments:
-                // 4 lanes per row, 8 rows per instruction.
-                __syncwarp();
+            for (int v4 = 0; v4 < 4; ++v4) {
+                o[v4 * 4 + 0] += gq[v4].x; o[v4 * 4 + 1] += gq[v4].y;
+                o[v4 * 4 + 2] += gq[v4].z; o[v4 * 4 + 3] += gq[v4].w;
+            }
+            if (c + 16 < BN) issue_group(c + 16);                // next group's loads overlap these stores
+            // A thread owns one ROW of the tile, so direct stores would scatter 16-byte pieces over 32 rows per
+            // instruction (measured: the epilogue was LSU-transaction-bound, 10.5k of 36k cycles per tile).  Stage the
+            // 32 x 16 block through shared memory (the pipeline stages are idle now) and write 64-byte row segments:
+            // 4 lanes per row, 8 rows per instruction.
+            __syncwarp();
 #pragma unroll
-                for (int v4 = 0; v4 < 4; ++v4)
-                    *reinterpret_cast<float4*>(stage + lane * 20 + v4 * 4) =
-                        make_float4(o[v4 * 4 + 0], o[v4 * 4 + 1], o[v4 * 4 + 2], o[v4 * 4 + 3]);
-                __syncwarp();
+            for (int v4 = 0; v4 < 4; ++v4)
+                *reinterpret_cast<float4*>(stage + lane * 20 + v4 * 4) =
+                    make_float4(o[v4 * 4 + 0], o[v4 * 4 + 1], o[v4 * 4 + 2], o[v4 * 4 + 3]);
+            __syncwarp();
 #pragma unroll
-                for (int t4 = 0; t4 < 4; ++t4) {
-                    const int f = t4 * 32 + lane, row = f >> 2, cq = f & 3;
-                    const int mr = m0 + h * 128 + q * 32 + row;
-                    if (mr < M && n0 + c + cq * 4 < N)          // N % 4 == 0; the last N tile may be partial
-                        *reinterpret_cast<float4*>(C + (size_t)mr * ldc + n0 + c + cq * 4) =
-                            *reinterpret_cast<const float4*>(stage + row * 20 + cq * 4);
-                }
+            for (int t4 = 0; t4 < 4; ++t4) {
+                const int f = t4 * 32 + lane, row = f >> 2, cq = f & 3;
+                const int mr = m0 + q * 32 + row;
+                if (mr < M && n0 + c + cq * 4 < N)          // N % 4 == 0; the last N tile may be partial
+                    *reinterpret_cast<float4*>(C + (size_t)mr * ldc + n0 + c + cq * 4) =
+                        *reinterpret_cast<const float4*>(stage + row * 20 + cq * 4);
             }
         }
     }
-#ifdef DIGAT_TC_TIMING
-    if (threadIdx.x == 64 && blockIdx.x == 2 && ((blockIdx.y % 997) == 5 || (gridDim.y < 6 && blockIdx.y == 1)))
-        printf("tile(%d,%d): epilogue done +%lld\n", blockIdx.x, blockIdx.y, clock64() - t_start);
-#endif
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 1) {
@@ -364,53 +332,39 @@ __global__ void split_tf32_kernel(const float* __restrict__ w, float* __restrict
     }
 }
 
-// bf16 planes of a weight for the correction products of the TF32+BF16 scheme (gemm_tcgen05_persistent.cuh):
-// hb = bf16(rna_tf32(W)) (stands in for W_hi in A_lo*W_hi), lb = bf16(W - rna_tf32(W)) (W_lo in A*W_lo).
-__global__ void split_bf16_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ hb, __nv_bfloat16* __restrict__ lb,
-                                  int64_t n) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) {
-        const float x = w[i];
-        const float h = to_tf32_rna(x);
-        hb[i] = __float2bfloat16_rn(h);
-        lb[i] = __float2bfloat16_rn(x - h);
-    }
-}
-
-template <int BN, int MH, bool SPLIT>
+template <int BN>
 inline int launch_tf32x3_cfg(const float* A, int lda, const float* W_hi, const float* W_lo, int ldw, const float* bias,
                              float* C, int ldc, int M, int N, int K, GroupBias gb, cudaStream_t st) {
-    using Cfg = TcCfg<BN, MH, SPLIT>;
+    using Cfg = TcCfg<BN>;
     CUtensorMap ma, mh, ml;
     int rc;
     if ((rc = make_tensor_map_2d(&ma, A, M, K, lda, Cfg::BM, kTcBK, CU_TENSOR_MAP_SWIZZLE_64B)) != DIGAT_OK) return rc;
     if ((rc = make_tensor_map_2d(&mh, W_hi, N, K, ldw, BN, kTcBK, CU_TENSOR_MAP_SWIZZLE_64B)) != DIGAT_OK) return rc;
     if ((rc = make_tensor_map_2d(&ml, W_lo, N, K, ldw, BN, kTcBK, CU_TENSOR_MAP_SWIZZLE_64B)) != DIGAT_OK) return rc;
-    if (int rc_ = ensure_dynamic_smem(gemm_tf32x3_kernel<BN, MH, SPLIT>, (size_t)(Cfg::SMEM))) return rc_;
+    if (int rc_ = ensure_dynamic_smem(gemm_tf32x3_kernel<BN>, (size_t)(Cfg::SMEM))) return rc_;
     dim3 grid((N + BN - 1) / BN, (M + Cfg::BM - 1) / Cfg::BM);
-    gemm_tf32x3_kernel<BN, MH, SPLIT><<<grid, kTcThreads, Cfg::SMEM, st>>>(ma, mh, ml, bias, C, ldc, M, N, K, gb);
+    gemm_tf32x3_kernel<BN><<<grid, kTcThreads, Cfg::SMEM, st>>>(ma, mh, ml, bias, C, ldc, M, N, K, gb);
     return check_launch("digat_linear_tf32x3");
 }
 
-static int g_tc_variant = 0;   // experiment switch (digat_debug_set_gemm_variant)
-static int g_tc_small_bn = 32, g_tc_small_rows = 1024;   // tile width for GEMMs of at most g_tc_small_rows rows (variants 10..13)
+// Row-group bias accepted by both tcgen05 projection GEMMs (digat_linear_tf32x3, digat_linear_bf16).
+inline int check_group_bias(const char* who, const GroupBias& gb, int N) {
+    DIGAT_REQUIRE(gb.ptr == nullptr || (gb.rows > 0 && gb.col0 >= 0 && gb.cols > 0 && gb.col0 + gb.cols <= N &&
+                                        (gb.col0 & 3) == 0 && (gb.cols & 3) == 0 && (gb.ld & 3) == 0 && gb.ld >= gb.cols &&
+                                        aligned16(gb.ptr)),
+                  "%s: bad row-group bias (col0/cols must be multiples of 4)", who);
+    return DIGAT_OK;
+}
 
 template <int BN>
-int launch_tf32x3_pair(const float* A, int lda, const float* W_hi, const float* W_lo, int ldw, const float* bias,
-                       float* C, int ldc, int M, int N, int K, GroupBias gb, cudaStream_t st);   // gemm_tcgen05_pair.cuh
-template <int BN>
 int launch_tf32x3_persistent(const float* A, int lda, const float* W_hi, const float* W_lo, int ldw, const float* bias,
-                             float* C, int ldc, int M, int N, int K, GroupBias gb, cudaStream_t st,
-                             const void* W_hb = nullptr, const void* W_lb = nullptr);   // gemm_tcgen05_persistent.cuh
+                             float* C, int ldc, int M, int N, int K, GroupBias gb, cudaStream_t st);   // gemm_tcgen05_persistent.cuh
 
 inline int launch_linear_tf32x3(const float* A, int lda, const float* W_hi, const float* W_lo, int ldw, const float* bias,
                                 float* C, int ldc, int M, int N, int K, GroupBias gb, cudaStream_t st) {
     if (M == 0) return DIGAT_OK;
     DIGAT_REQUIRE(A && W_hi && W_lo && C, "digat_linear_tf32x3: null pointer");
-    DIGAT_REQUIRE(gb.ptr == nullptr || (gb.rows > 0 && gb.col0 >= 0 && gb.cols > 0 && gb.col0 + gb.cols <= N &&
-                                        (gb.col0 & 3) == 0 && (gb.cols & 3) == 0 && (gb.ld & 3) == 0 && gb.ld >= gb.cols &&
-                                        aligned16(gb.ptr)),
-                  "digat_linear_tf32x3: bad row-group bias (col0/cols must be multiples of 4)");
+    if (int rc_ = check_group_bias("digat_linear_tf32x3", gb, N)) return rc_;
     DIGAT_REQUIRE(M >= 0 && N > 0 && K > 0, "digat_linear_tf32x3: bad shape M=%d N=%d K=%d", M, N, K);
     DIGAT_REQUIRE((K & 3) == 0 && (lda & 3) == 0 && (ldw & 3) == 0 && (ldc & 3) == 0,
                   "digat_linear_tf32x3: K, lda, ldw, ldc must be multiples of 4");
@@ -418,47 +372,26 @@ inline int launch_linear_tf32x3(const float* A, int lda, const float* W_hi, cons
     DIGAT_REQUIRE(aligned16(A) && aligned16(W_hi) && aligned16(W_lo) && aligned16(C) && (!bias || aligned16(bias)),
                   "digat_linear_tf32x3: pointers must be 16-byte aligned");
     DIGAT_REQUIRE(N % 16 == 0, "digat_linear_tf32x3: N=%d must be a multiple of 16", N);
-    if (M == 0) return DIGAT_OK;
     DIGAT_REQUIRE(gb.kbatches >= 1, "digat_linear_tf32x3: bad split-K batch count");
-    if (gb.out_rows != nullptr || gb.kbatches > 1) {      // row scatter / split-K live in the persistent kernel only
-        DIGAT_REQUIRE(N <= 1280, "digat_linear_tf32x3: c_row_index needs N <= 1280 (N=%d)", N);
+    const bool scatter = gb.out_rows != nullptr || gb.kbatches > 1;    // row scatter / split-K live in the persistent kernel only
+    if (scatter) DIGAT_REQUIRE(N <= 1280, "digat_linear_tf32x3: c_row_index needs N <= 1280 (N=%d)", N);
+    const bool big = M > kTcBigRows;
+    // Large M: persistent 128 x 240 tiles, or 208-wide ones for widths that 240 does not divide (N = 400: featureAffine)
+    // when they waste < 10 % of the MMA columns (400 -> 2 x 208 = 4 %; the 128-wide tiles below compute 512 columns = 28 %).
+    if (scatter || (big && N <= 1280 && (N % 240 == 0 || ((N + 207) / 208) * 208 * 10 < N * 11))) {
         if (N % 240 == 0) return launch_tf32x3_persistent<240>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
         return launch_tf32x3_persistent<208>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
     }
-    // variant 0 (default): one 128-row half per CTA, separate main / correction accumulators (most accurate);
-    // variant 1: two halves per CTA for M > 16384, single accumulator (half the W traffic per flop, less accurate).
-    const int variant = g_tc_variant;
-    const bool big = M > 16384;
-    if (variant == 0 && big && N % 240 == 0 && N <= 1280) // persistent 128 x 240 tiles (variant 4 = one tile per CTA)
-        return launch_tf32x3_persistent<240>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-    // widths that 240 does not divide (N = 400: featureAffine): 208-wide persistent tiles when they waste < 10 % of the
-    // MMA columns (400 -> 2 x 208 = 4 %; the 128-wide fallback below computes 512 columns = 28 %)
-    if (variant == 0 && big && N <= 1280 && ((N + 207) / 208) * 208 * 10 < N * 11)
-        return launch_tf32x3_persistent<208>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-    if (variant == 3 && N % 240 == 0)                    // 2-CTA (cta_group::2) 256 x 240 tiles
-        return launch_tf32x3_pair<240>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
     // a few hundred rows (the context projections of a training step, M = batch): three 128-row tiles x N/128 columns
     // would occupy a dozen SMs, each pulling its whole A panel and 2 W planes through one SM's ingest; narrow tiles
     // spread the same MMAs over N/32 times as many SMs (results are bit-identical: the k order per element is unchanged)
-    if ((variant == 0 || variant == 4) && M <= g_tc_small_rows && g_tc_small_bn != 128) {
-        if (g_tc_small_bn == 64) return launch_tf32x3_cfg<64, 1, true>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-        if (g_tc_small_bn == 16) return launch_tf32x3_cfg<16, 1, true>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-        return launch_tf32x3_cfg<32, 1, true>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-    }
-    // small problems (few tiles) and odd widths: 128-wide tiles, two CTAs per SM (measured 1.45x faster at M = 4096);
-    // the last N tile may be partial.  Large M keeps the 240-wide tile (fewer re-reads of A: measured 185 vs 158 TFLOP/s).
-    if (variant == 2 || N % 80 != 0 || ((variant == 0 || variant == 4) && (!big || (N % 240 != 0 && N % 160 != 0))))
-        return launch_tf32x3_cfg<128, 1, true>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
-#define DIGAT_TC_DISPATCH(BN_)                                                                                      \
-    do {                                                                                                            \
-        if (variant == 1 && big) return launch_tf32x3_cfg<BN_, 2, false>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st); \
-        if (variant == 1) return launch_tf32x3_cfg<BN_, 1, false>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);        \
-        return launch_tf32x3_cfg<BN_, 1, true>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);                 \
-    } while (0)
-    if (N % 240 == 0) DIGAT_TC_DISPATCH(240);
-    if (N % 160 == 0) DIGAT_TC_DISPATCH(160);
-    DIGAT_TC_DISPATCH(80);
-#undef DIGAT_TC_DISPATCH
+    if (M <= kTcSmallRows) return launch_tf32x3_cfg<32>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
+    // Large M keeps a wide tile (fewer re-reads of A: measured 185 vs 158 TFLOP/s at 240 against 128).  Small problems
+    // (few tiles) and the other widths: 128-wide tiles, two CTAs per SM (measured 1.45x faster at M = 4096); the last N
+    // tile may be partial.
+    if (big && N % 240 == 0) return launch_tf32x3_cfg<240>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
+    if (big && N % 160 == 0) return launch_tf32x3_cfg<160>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
+    return launch_tf32x3_cfg<128>(A, lda, W_hi, W_lo, ldw, bias, C, ldc, M, N, K, gb, st);
 }
 
 }  // namespace digat

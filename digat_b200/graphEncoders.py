@@ -85,11 +85,11 @@ class PackedWeight:
     """A projection weight in kernel layout: fp32 [N,K] (nn.Linear layout) plus, when the tcgen05 GEMM can take it
     (N % 16 == 0, K % 4 == 0), its two TF32 planes hi = rna_tf32(W), lo = rna_tf32(W - hi) (digat_split_tf32).
     bf16=True adds wb = bf16_rn(W): linear() then runs this weight's products on the BF16 GEMM (digat_linear_bf16)."""
-    __slots__ = ('w', 'hi', 'lo', 'hb', 'lb', 'wb')
+    __slots__ = ('w', 'hi', 'lo', 'wb')
 
     def __init__(self, w, bf16=False):
         self.w = w.detach().float().contiguous()
-        self.hi = self.lo = self.hb = self.lb = self.wb = None
+        self.hi = self.lo = self.wb = None
         if bf16:
             if self.w.shape[0] % 16 != 0 or self.w.shape[0] > 1280 or self.w.shape[1] % 8 != 0:
                 raise RuntimeError('PackedWeight: the BF16 GEMM needs N %% 16 == 0, N <= 1280, K %% 8 == 0 (got %s)'
@@ -99,24 +99,10 @@ class PackedWeight:
             self.hi, self.lo = torch.empty_like(self.w), torch.empty_like(self.w)
             _lib.call('digat_split_tf32', self.w.data_ptr(), self.hi.data_ptr(), self.lo.data_ptr(), self.w.numel(),
                       _stream())
-            if GEMM_BF16_CORRECTIONS and self.w.shape[1] % 8 == 0 and self.w.shape[0] <= 1280:
-                # bf16 planes of the correction products (digat_linear_tf32_bf16c): bf16(rna_tf32(W)), bf16(W - rna_tf32(W))
-                self.hb = torch.empty(self.w.shape, dtype=torch.bfloat16, device=self.w.device)
-                self.lb = torch.empty_like(self.hb)
-                _lib.call('digat_split_bf16', self.w.data_ptr(), self.hb.data_ptr(), self.lb.data_ptr(), self.w.numel(),
-                          _stream())
 
 
 # rows below which the exact-fp32 CUDA-core GEMM is used (a 128-row tensor-core tile would be mostly padding)
 TENSOR_CORE_MIN_ROWS = 256
-# Optional: large projections (persistent kernel, dense row count >= BF16C_MIN_ROWS) run the two correction products of the
-# 3xTF32 scheme as BF16 MMAs (digat_linear_tf32_bf16c: 4 instead of 6 TF32-MMA times per k-block).  Validated (the L=7
-# golden case x64 and the sampled bench batches stay inside the 1e-5 gate with it on), but OFF by default: the GEMM is bound
-# by the bytes each SM takes in per k-block, not by the tensor pipe, so it buys 3.5 % on the GEMM (~1 % of a step,
-# profiles/r2_gemm_variants.txt) while a size-dependent scheme would end the bit-identity of the shared-user-graph and the
-# expanded scoring paths (their layer-0 projections have different row counts).
-GEMM_BF16_CORRECTIONS = False
-BF16C_MIN_ROWS = 16385
 
 
 def linear(A, W, bias=None, relu=False, M=None, K=None, lda=None, out=None, group_bias=None, group_rows=1,
@@ -141,29 +127,15 @@ def linear(A, W, bias=None, relu=False, M=None, K=None, lda=None, out=None, grou
         out = torch.empty((M, N), device=A.device, dtype=torch.float32)
     gcols = 0 if group_bias is None else group_bias.shape[1]
     gld = 0 if group_bias is None else group_bias.stride(0)
-    # (the scheme is chosen from the DENSE row count of the output, so a pruned / row-scattered call and its un-pruned
-    # counterpart take the same arithmetic and stay bit-identical)
-    m_dense = out.shape[0] if c_rows is not None else M
-    bf16c = GEMM_BF16_CORRECTIONS and isinstance(W, PackedWeight) and W.hb is not None and m_dense >= BF16C_MIN_ROWS and \
-        (K & 7) == 0 and not relu
     if bf16:                                                            # every M, with or without c_rows
         _lib.call('digat_linear_bf16', A.data_ptr(), lda, W.wb.data_ptr(), W.wb.stride(0), _ptr(bias), out.data_ptr(),
                   out.stride(0), M, N, K, _ptr(group_bias), group_rows, group_col0, gcols, gld, _ptr(c_rows), _stream())
     elif c_rows is not None:
         if not (isinstance(W, PackedWeight) and W.hi is not None) or relu:
             raise RuntimeError('linear: c_rows needs a PackedWeight with TF32 planes and no relu')
-        if bf16c:
-            _lib.call('digat_linear_tf32_bf16c', A.data_ptr(), lda, W.hi.data_ptr(), W.hb.data_ptr(), W.lb.data_ptr(),
-                      w.stride(0), _ptr(bias), out.data_ptr(), out.stride(0), M, N, K, _ptr(group_bias), group_rows,
-                      group_col0, gcols, gld, c_rows.data_ptr(), _stream())
-        else:
-            _lib.call('digat_linear_tf32x3', A.data_ptr(), lda, W.hi.data_ptr(), W.lo.data_ptr(), w.stride(0), _ptr(bias),
-                      out.data_ptr(), out.stride(0), M, N, K, _ptr(group_bias), group_rows, group_col0, gcols, gld,
-                      c_rows.data_ptr(), _stream())
-    elif bf16c:
-        _lib.call('digat_linear_tf32_bf16c', A.data_ptr(), lda, W.hi.data_ptr(), W.hb.data_ptr(), W.lb.data_ptr(),
-                  w.stride(0), _ptr(bias), out.data_ptr(), out.stride(0), M, N, K, _ptr(group_bias), group_rows,
-                  group_col0, gcols, gld, 0, _stream())
+        _lib.call('digat_linear_tf32x3', A.data_ptr(), lda, W.hi.data_ptr(), W.lo.data_ptr(), w.stride(0), _ptr(bias),
+                  out.data_ptr(), out.stride(0), M, N, K, _ptr(group_bias), group_rows, group_col0, gcols, gld,
+                  c_rows.data_ptr(), _stream())
     elif isinstance(W, PackedWeight) and W.hi is not None and M >= TENSOR_CORE_MIN_ROWS and not relu:
         _lib.call('digat_linear_tf32x3', A.data_ptr(), lda, W.hi.data_ptr(), W.lo.data_ptr(), w.stride(0), _ptr(bias),
                   out.data_ptr(), out.stride(0), M, N, K, _ptr(group_bias), group_rows, group_col0, gcols, gld, 0,

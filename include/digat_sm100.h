@@ -14,7 +14,7 @@
  *   - return value: 0 on success, <0 on failure (DIGAT_E_*); digat_last_error() gives the message of the
  *     last failure on the calling thread.  Nothing throws or exits across this boundary.
  *   - entry points are re-entrant (process-wide mutable state: cached device properties, a mutex-guarded TMA
- *     descriptor cache, and the digat_debug_set_* experiment switches, which nothing on the reference path sets);
+ *     descriptor cache, and the digat_debug_set_layer_mode test switch, which nothing on the reference path sets);
  *     there is no CPU fallback: without an sm_100 device every compute call fails.
  */
 #ifndef DIGAT_SM100_H
@@ -31,7 +31,7 @@ extern "C" {
 #define DIGAT_E_CUDA        -2   /* a CUDA runtime/driver call or a launch failed */
 #define DIGAT_E_UNSUPPORTED -3   /* device is not sm_100 */
 
-#define DIGAT_ABI_VERSION 6
+#define DIGAT_ABI_VERSION 7
 
 int         digat_abi_version(void);
 const char* digat_last_error(void);
@@ -68,7 +68,7 @@ int digat_split_tf32(const float* W, float* W_hi, float* W_lo, int64_t count, vo
 /* tcgen05 tensor-core GEMM, operands fed by TMA, fp32 accumulators in TMEM, fp32-level accuracy by 3xTF32 error
  * compensation: C = A_hi*W_hi + A_lo*W_hi + A_hi*W_lo (+ bias).  A is plain fp32 and is split into its TF32 planes
  * on the fly inside the kernel; W_hi / W_lo come from digat_split_tf32 (same ldw).
- * Requires K % 4 == 0, N % 80 == 0, lda/ldw/ldc % 4 == 0.  Replaces the three node projections h, K1, K2 of one
+ * Requires K % 4 == 0, N % 16 == 0, lda/ldw/ldc % 4 == 0.  Replaces the three node projections h, K1, K2 of one
  * layer as ONE GEMM against the stacked [3D, D] weight (graphEncoders.py:146-148 / 166-168).
  * c_row_index (may be NULL; ascending int32 [M]): row scatter -- product row m is written to row c_row_index[m] of C
  * and takes the row-group bias of that row.  A then holds only the node rows worth projecting (see
@@ -78,18 +78,6 @@ int digat_linear_tf32x3(const float* A, int lda, const float* W_hi, const float*
                         const float* bias, float* C, int ldc, int M, int N, int K,
                         const float* group_bias, int group_rows, int group_col0, int group_cols, int group_ld,
                         const int32_t* c_row_index, void* stream);
-
-/* TF32 + BF16-correction form of the projection GEMM (large M; persistent tcgen05 kernel):
- *   C = A_hi*W_hi [TF32 MMAs on the raw fp32 A]  +  bf16(A)*bf16(W_lo)  +  bf16(A_lo)*bf16(W_hi)  [BF16 MMAs]
- * The two correction products are ~2^-11 of the result and need only ~9 good bits, so they run as BF16 MMAs at twice the
- * TF32 rate: 4 instead of 6 TF32-MMA times per k-block at the same fp32-level accuracy (measured in tests/test_gpu_gemm.py).
- * W_hi = rna_tf32(W) (digat_split_tf32); W_hb = bf16(W_hi), W_lb = bf16(W - W_hi) (digat_split_bf16), all with row pitch
- * ldw elements.  Same bias / row-group bias / row scatter semantics as digat_linear_tf32x3.  K, ldw % 8 == 0, N <= 1280. */
-int digat_split_bf16(const float* W, void* W_hb, void* W_lb, int64_t count, void* stream);
-int digat_linear_tf32_bf16c(const float* A, int lda, const float* W_hi, const void* W_hb, const void* W_lb, int ldw,
-                            const float* bias, float* C, int ldc, int M, int N, int K,
-                            const float* group_bias, int group_rows, int group_col0, int group_cols, int group_ld,
-                            const int32_t* c_row_index, void* stream);
 
 /* C = bf16_rn(A) * W_b^T (+bias)(+row-group bias), fp32 accumulation.  W_b = bf16_rn(W) [N,K] (row pitch ldw).
  * Same bias / group-bias / c_row_index semantics and alignment rules as digat_linear_tf32x3; K, ldw % 8 == 0, N <= 1280.
@@ -108,10 +96,6 @@ int digat_linear_tf32x3_splitk(const float* A, int lda, const float* W_hi, const
                                float* C, int ldc, int M, int N, int K, int kbatches, int64_t c_batch_stride,
                                void* stream);
 
-/* Tuning/experiment switch for digat_linear_tf32x3 (0 = default).  Not part of the reference path.
- * 0-4: tile variants of the non-persistent kernel; 6/7/8: persistent kernel as independent CTAs (default) / W multicast over a
- * CTA pair / 2-CTA MMA; 10-13: tile width of GEMMs with at most 1024 rows = 128 (off) / 64 / 32 (default) / 16. */
-int digat_debug_set_gemm_variant(int variant);
 /* digat_graph_layer_fwd kernel choice: 0 = auto (edge-driven kernel when a CTA owns one graph and no training extras are
  * requested, dense kernel otherwise), 1 = always dense, 2 = always edge-driven (inference).  For tests / profiling. */
 int digat_debug_set_layer_mode(int mode);

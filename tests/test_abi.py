@@ -16,7 +16,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r'\b(digat_[a-z0-9_]+)\s*\(', src)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_7():
     from digat_b200 import _lib
     lib = ctypes.CDLL(_lib.LIB_PATH)
     names = _declared_symbols()
@@ -25,7 +25,7 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, n), 'libdigat_sm100.so does not export ' + n
     bound = set(_lib.SIGNATURES) | {'digat_last_error'}
     assert set(names) == bound, 'ctypes SIGNATURES out of sync with the header: %s' % (set(names) ^ bound)
-    assert _lib.load().digat_abi_version() == 6
+    assert _lib.load().digat_abi_version() == 7
 
 
 def test_no_gpu_fails_loudly():

@@ -40,7 +40,8 @@ def test_split_planes_are_exact_tf32():
 
 
 @pytest.mark.parametrize('M,N,K', [(128, 240, 16), (128, 80, 400), (256, 1200, 400), (1000, 400, 400),
-                                   (4096, 400, 800), (20000, 1200, 400), (69632, 1200, 400), (16385, 800, 400)])
+                                   (4096, 400, 800), (20000, 1200, 400), (69632, 1200, 400), (16385, 800, 400),
+                                   (20000, 640, 400), (20000, 1440, 400)])
 def test_tf32x3_matches_fp64(M, N, K):
     g = torch.Generator().manual_seed(M + N + K)
     A = torch.randn(M, K, generator=g)
@@ -90,30 +91,6 @@ def test_group_bias_folds_k3_into_K1_block(M, n):
     assert torch.equal(out, expect)
 
 
-def test_tf32_bf16_correction_gemm_matches_fp64():
-    """digat_linear_tf32_bf16c (experimental scheme: TF32 main product, BF16 correction products) keeps fp32-level
-    accuracy, with bias, row-group bias and a partial last N tile."""
-    from digat_b200 import _lib
-    g = torch.Generator().manual_seed(3)
-    for (M, N, K) in [(20000, 1200, 400), (5000, 400, 800), (300, 240, 64)]:
-        A = torch.randn(M, K, generator=g).cuda()
-        W = (torch.randn(N, K, generator=g) * 0.05).cuda()
-        b = torch.randn(N, generator=g).cuda()
-        gbias = torch.randn((M + 67) // 68, 400 if N >= 400 else 80, generator=g).cuda()
-        hi, lo = _split(W)
-        hb = torch.empty(W.shape, dtype=torch.bfloat16, device='cuda')
-        lb = torch.empty_like(hb)
-        st = torch.cuda.current_stream().cuda_stream
-        _lib.call('digat_split_bf16', W.data_ptr(), hb.data_ptr(), lb.data_ptr(), W.numel(), st)
-        C = torch.full((M, N), float('nan'), device='cuda')
-        _lib.call('digat_linear_tf32_bf16c', A.data_ptr(), K, hi.data_ptr(), hb.data_ptr(), lb.data_ptr(), K, b.data_ptr(),
-                  C.data_ptr(), N, M, N, K, gbias.data_ptr(), 68, 0, gbias.shape[1], gbias.shape[1], 0, st)
-        torch.cuda.synchronize()
-        ref = A.double().cpu() @ W.double().cpu().t() + b.double().cpu()
-        ref[:, :gbias.shape[1]] += gbias.double().cpu().repeat_interleave(68, dim=0)[:M]
-        assert rel_err(C.cpu().numpy(), ref.numpy()) < 4e-6
-
-
 @pytest.mark.parametrize('M,N,K', [(300, 64, 64), (1000, 256, 256), (20000, 512, 128), (40000, 128, 512), (700, 48, 32)])
 def test_tf32x3_widths_that_80_does_not_divide(M, N, K):
     """news_embedding_dim values such as 64 / 128 / 256 / 512 (ADVICE r1): partial last N tiles on every tile variant."""
@@ -147,9 +124,10 @@ def test_linear_backward_other_embedding_dims(M, D):
 
 
 @pytest.mark.parametrize('M,N,K', [(100000, 1200, 400), (77824, 400, 400), (136000 + 77, 1200, 400), (30000, 480, 96)])
-def test_w_multicast_cluster_kernel_is_bit_identical(M, N, K):
-    """The cluster variant of the persistent kernel (two CTAs share the W tile by TMA multicast) does the same arithmetic per
-    output element as independent CTAs: bit-identical, including the odd M-block tail, bias, row-group bias and row scatter."""
+def test_persistent_kernel_row_scatter_is_dense_product_plus_group_bias(M, N, K):
+    """The persistent kernel with bias, row-group bias, an odd M-block tail and ascending row scatter: row m of the product
+    lands in C[rows[m]] as the dense product D[m] of the same call without scatter or group bias, plus the group bias of
+    row rows[m] in one fp32 add on the bias columns, bit for bit; the rows of C that are not listed stay untouched."""
     from digat_b200 import _lib
     g = torch.Generator().manual_seed(M + N)
     A = torch.randn(M, K, generator=g).cuda()
@@ -160,59 +138,24 @@ def test_w_multicast_cluster_kernel_is_bit_identical(M, N, K):
     rows = torch.sort(torch.randperm(2 * M, generator=g)[:M]).values.to(torch.int32).cuda()      # ascending scatter targets
     hi, lo = _split(W)
     st = torch.cuda.current_stream().cuda_stream
-    out = {}
-    try:
-        for variant in (6, 7, 8):                                         # 6 = independent CTAs, 7 = W multicast, 8 = 2-CTA MMA
-            _lib.call('digat_debug_set_gemm_variant', variant)
-            C = torch.zeros((2 * M, N), device='cuda')
-            _lib.call('digat_linear_tf32x3', A.data_ptr(), K, hi.data_ptr(), lo.data_ptr(), K, bias.data_ptr(), C.data_ptr(), N,
-                      M, N, K, gbias.data_ptr(), 68, 0, gcols, gcols, rows.data_ptr(), st)
-            D = torch.zeros((M, N), device='cuda')
-            _lib.call('digat_linear_tf32x3', A.data_ptr(), K, hi.data_ptr(), lo.data_ptr(), K, bias.data_ptr(), D.data_ptr(), N,
-                      M, N, K, 0, 1, 0, 0, 0, 0, st)
-            torch.cuda.synchronize()
-            out[variant] = (C, D)
-    finally:
-        _lib.call('digat_debug_set_gemm_variant', 6)
-    assert torch.equal(out[6][0], out[7][0]) and torch.equal(out[6][1], out[7][1])
-    # the 2-CTA MMA issues the correction products in another order (no early raw-A issue): equal to rounding, not bitwise
-    for k in (0, 1):
-        assert float((out[6][k] - out[8][k]).abs().max()) <= 2e-6 * float(out[6][k].abs().max())
-    sel = torch.randperm(M, generator=g)[:256]
-    ref = A[sel].double().cpu() @ W.double().cpu().t() + bias.double().cpu()
-    assert rel_err(out[8][1][sel].cpu().numpy(), ref.numpy()) < 4e-6
-
-
-def test_bf16_correction_scheme_with_multicast_and_scatter():
-    """digat_linear_tf32_bf16c on the cluster kernel (the hot-path configuration): vs fp64, and cluster on == off."""
-    from digat_b200 import _lib
-    g = torch.Generator().manual_seed(9)
-    M, N, K = 120000, 1200, 400
-    A = torch.randn(M, K, generator=g).cuda()
-    W = (torch.randn(N, K, generator=g) * 0.05).cuda()
-    b = torch.randn(N, generator=g).cuda()
-    hi, lo = _split(W)
-    hb = torch.empty(W.shape, dtype=torch.bfloat16, device='cuda')
-    lb = torch.empty_like(hb)
-    st = torch.cuda.current_stream().cuda_stream
-    _lib.call('digat_split_bf16', W.data_ptr(), hb.data_ptr(), lb.data_ptr(), W.numel(), st)
-    rows = torch.sort(torch.randperm(2 * M, generator=g)[:M]).values.to(torch.int32).cuda()
-    out = {}
-    try:
-        for variant in (6, 7, 8):
-            _lib.call('digat_debug_set_gemm_variant', variant)
-            C = torch.zeros((2 * M, N), device='cuda')
-            _lib.call('digat_linear_tf32_bf16c', A.data_ptr(), K, hi.data_ptr(), hb.data_ptr(), lb.data_ptr(), K, b.data_ptr(),
-                      C.data_ptr(), N, M, N, K, 0, 1, 0, 0, 0, rows.data_ptr(), st)
-            torch.cuda.synchronize()
-            out[variant] = C
-    finally:
-        _lib.call('digat_debug_set_gemm_variant', 6)
-    assert torch.equal(out[6], out[7])
-    assert float((out[6] - out[8]).abs().max()) <= 2e-6 * float(out[6].abs().max())
-    sel = torch.randperm(M, generator=g)[:256]
-    ref = A[sel].double().cpu() @ W.double().cpu().t() + b.double().cpu()
-    assert rel_err(out[7][rows[sel].long()].cpu().numpy(), ref.numpy()) < 4e-6
+    C = torch.zeros((2 * M, N), device='cuda')
+    _lib.call('digat_linear_tf32x3', A.data_ptr(), K, hi.data_ptr(), lo.data_ptr(), K, bias.data_ptr(), C.data_ptr(), N,
+              M, N, K, gbias.data_ptr(), 68, 0, gcols, gcols, rows.data_ptr(), st)
+    D = torch.full((M, N), float('nan'), device='cuda')
+    _lib.call('digat_linear_tf32x3', A.data_ptr(), K, hi.data_ptr(), lo.data_ptr(), K, bias.data_ptr(), D.data_ptr(), N,
+              M, N, K, 0, 1, 0, 0, 0, 0, st)
+    torch.cuda.synchronize()
+    r = rows.long()
+    expect = D.clone()
+    expect[:, :gcols] = D[:, :gcols] + gbias[r // 68]
+    assert torch.equal(C[r], expect)
+    listed = torch.zeros(2 * M, dtype=torch.bool, device='cuda')
+    listed[r] = True
+    assert int(torch.count_nonzero(C[~listed])) == 0
+    sel = torch.randperm(M, generator=g)[:256].cuda()
+    ref = A[sel].double() @ W.double().t() + bias.double()
+    ref[:, :gcols] += gbias[r[sel] // 68].double()
+    assert rel_err(C[r[sel]].cpu().numpy(), ref.cpu().numpy()) < 4e-6
 
 
 @pytest.mark.parametrize('M,N,K', [(320, 400, 400), (320, 800, 400), (7, 36, 52), (1, 4, 4), (1000, 400, 1200), (33, 400, 68)])
