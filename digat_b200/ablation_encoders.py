@@ -15,7 +15,9 @@ A vanilla-GAT layer is a degenerate Eq. (8): ``digat_gat_layer_fwd`` runs the ed
 formed by one add of two per-node dot products, streaming h only.  All five TRAIN through autograd_ops.encode_with_grad
 (``forward`` with gradients enabled): ``wo_SA`` / ``Seq_SA`` as their own schedules of the DIGAT layer and contexts, the
 vanilla-GAT layers through GATLayerFn (digat_gat_layer_train_fwd / digat_gat_layer_bwd_csr); ``inference`` is a no-grad path.  Node pruning is off here
-(every node is projected and evaluated): these are not the benchmarked path."""
+(every node is projected and evaluated).  Each encoder also has a scoring schedule for scoring.Scorer (``_encode``,
+``_news_cache``, ``SCORE_NEWS_NODES``): the parts that do not depend on the pair run once per news or once per behaviour
+(DESIGN.md section 4.6)."""
 import torch
 import torch.nn as nn
 
@@ -183,6 +185,44 @@ class _AblationEncoder(DIGAT):
             c_u, k3u = self._user_ctx(w, Xu, Mc, ci, c_n, i + 1, ctx_in=c_u)
         return c_n, c_u
 
+    # ---------------------------------------------------------------------------------- scoring schedules
+    # scoring.Scorer calls _encode with DIGAT's contract: when share [B] int32 is given, Xu / Au / ci are per-BEHAVIOUR
+    # tables and pair b uses entry share[b]; c_n holds each pair's rows of _news_cache.  Every part of a schedule that does
+    # not depend on the pair runs once per behaviour (user side) or once per news (the cache).  Without share every step
+    # runs per pair; the results are the same to the bit (the same rows go through the same kernels).  The pruning lists
+    # stay None: these encoders evaluate every node.
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        raise RuntimeError('%s has no scoring schedule' % type(self).__name__)
+
+    def _gat_contexts(self, w, Xn, An, Mn):
+        """c_n^(0..L) [B, L+1, D] of a vanilla-GAT news graph: its layers never read the user side (reference :494-503),
+        so every news context of the schedule depends on the candidate news only."""
+        cs = [self._news_ctx(w, Xn, Mn)]
+        for i in range(self.graph_depth):
+            Xn = self._gat(w, 'news', i, Xn, An)
+            cs.append(self._news_ctx(w, Xn, Mn, ctx_in=cs[-1]))
+        return torch.stack(cs, 1)
+
+    def _gat_stack(self, w, g, X, adj):
+        """[X, layer 0 output, ..., layer L-1 output] of a vanilla-GAT graph (per behaviour when X / adj are)."""
+        Xs = [X]
+        for i in range(self.graph_depth):
+            Xs.append(self._gat(w, g, i, Xs[-1], adj))
+        return Xs
+
+    def _user_digat_prep(self, Au, ci, share, first_rows):
+        """(CSR record of the user graphs, per-pair category ids) for the DIGAT user layers of a scoring schedule: the
+        record follows the adjacency (one per behaviour when shared); from layer 1 on every pair owns its user nodes."""
+        csr = self._user_csr(Au, None, share, first_rows)[0] if self.graph_depth else None
+        return csr, (ci if share is None else ci.index_select(0, share.long()))
+
+    def _user_digat_layer(self, w, i, Xu, Au, ctx, k3, share, csr):
+        """DIGAT user layer i of a scoring schedule (k3 None: formed here from ctx).  Layer 0 reads the per-behaviour node
+        table through share, so its projection runs once per behaviour (as DIGAT's layer 0); later layers run per pair on
+        the per-behaviour adjacency."""
+        return self._layer(w, 'user', i, Xu, Au, ctx, k3=k3, share=share if i == 0 else None,
+                           adj_index=share if i > 0 else None, csr=csr, csr_last=csr)[0]
+
     # ---------------------------------------------------------------------------------- reference API
     def _no_grad_only(self, *tensors):
         if torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters())
@@ -246,6 +286,22 @@ class wo_SA(_AblationEncoder):
     def compute_news_graph_context(self, news_graph_embeddings, news_graph_mask):
         raise Exception('wo_SA has no news-graph context (reference graphEncoders.py:201-295)')
 
+    SCORE_NEWS_NODES = 'first'   # the news side is the candidate's own embedding: nothing to cache
+
+    def _news_cache(self, w, Xn, An, Mn):
+        return None
+
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        """Scoring schedule of _run: k3 = ffn3_i(candidate) per pair, the user stack after layer 0 per pair."""
+        cand = Xn[:, 0, :].contiguous()
+        csr, ci_pair = self._user_digat_prep(Au, ci, share, first_rows)
+        for i in range(self.graph_depth):
+            Xu = self._user_digat_layer(w, i, Xu, Au, cand, None, share, csr)
+        per_beh = share is not None and self.graph_depth == 0                 # no layer: the nodes are still per behaviour
+        c_u, _ = self._user_ctx(w, Xu, Mc, ci if per_beh else ci_pair, cand, self.graph_depth,
+                                src_index=share if per_beh else None)
+        return cand, c_u
+
     def _run(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n):
         cand = Xn[:, 0, :].contiguous()                         # single_candidate_news_representation (:281 / :290)
         for i in range(self.graph_depth):
@@ -270,6 +326,20 @@ class Seq_SA(_AblationEncoder):
         """util.py:48 calls this instead of compute_news_graph_context (same arithmetic, reference :342-347)."""
         return DIGAT.compute_news_graph_context(self, news_graph_embeddings, news_graph_mask)
 
+    SCORE_NEWS_NODES = 'none'    # the news side is the sequence context, cached per news (DIGAT._news_cache: the same
+                                 # arithmetic as compute_news_sequence_context)
+
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        """Scoring schedule of _run: c_n is fixed over the layers; the user side as DIGAT's (layer 0 per behaviour)."""
+        if c_n is None:
+            c_n = self._news_ctx(w, Xn, Mn)
+        csr, ci_pair = self._user_digat_prep(Au, ci, share, first_rows)
+        c_u, k3u = self._user_ctx(w, Xu, Mc, ci, c_n, 0, src_index=share)
+        for i in range(self.graph_depth):
+            Xu = self._user_digat_layer(w, i, Xu, Au, c_n, k3u, share, csr)
+            c_u, k3u = self._user_ctx(w, Xu, Mc, ci_pair, c_n, i + 1, ctx_in=c_u)
+        return c_n, c_u
+
     def _run(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n):
         if c_n is None:
             c_n = self._news_ctx(w, Xn, Mn)
@@ -285,6 +355,19 @@ class wo_interaction(_AblationEncoder):
     NEWS_LAYER = 'gat'
     USER_LAYER = 'gat'
     TRAIN_SCHEDULE = 'digat'     # the dual-graph schedule; the layer kinds come from NEWS_LAYER / USER_LAYER
+    SCORE_NEWS_NODES = 'none'    # the whole news side is cached per news
+
+    def _news_cache(self, w, Xn, An, Mn):
+        return self._gat_contexts(w, Xn, An, Mn)
+
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        """Scoring schedule of _run: the user GAT stack runs once per behaviour, so per pair only the L+1 user contexts
+        remain (they read c_n^(j), the cached news contexts [B, L+1, D])."""
+        cs = self._news_cache(w, Xn, An, Mn) if c_n is None else c_n
+        c_u = None
+        for j, Xj in enumerate(self._gat_stack(w, 'user', Xu, Au)):
+            c_u, _ = self._user_ctx(w, Xj, Mc, ci, cs[:, j], j, ctx_in=c_u, src_index=share)
+        return cs[:, self.graph_depth].contiguous(), c_u
 
 
 class News_graph_wo_inter(_AblationEncoder):
@@ -292,6 +375,21 @@ class News_graph_wo_inter(_AblationEncoder):
     NEWS_LAYER = 'gat'
     USER_LAYER = 'digat'
     TRAIN_SCHEDULE = 'digat'
+    SCORE_NEWS_NODES = 'none'    # the whole news side is cached per news
+
+    def _news_cache(self, w, Xn, An, Mn):
+        return self._gat_contexts(w, Xn, An, Mn)
+
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        """Scoring schedule of _run: the news contexts c_n^(j) come from the cache [B, L+1, D]; the user side as DIGAT's
+        with k3 = ffn3(c_n^(i)) (layer 0 per behaviour)."""
+        cs = self._news_cache(w, Xn, An, Mn) if c_n is None else c_n
+        csr, ci_pair = self._user_digat_prep(Au, ci, share, first_rows)
+        c_u, k3u = self._user_ctx(w, Xu, Mc, ci, cs[:, 0], 0, src_index=share)
+        for i in range(self.graph_depth):
+            Xu = self._user_digat_layer(w, i, Xu, Au, None, k3u, share, csr)
+            c_u, k3u = self._user_ctx(w, Xu, Mc, ci_pair, cs[:, i + 1], i + 1, ctx_in=c_u)
+        return cs[:, self.graph_depth].contiguous(), c_u
 
 
 class User_graph_wo_inter(_AblationEncoder):
@@ -299,6 +397,19 @@ class User_graph_wo_inter(_AblationEncoder):
     NEWS_LAYER = 'digat'
     USER_LAYER = 'gat'
     TRAIN_SCHEDULE = 'digat'
+
+    def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
+        """Scoring schedule of _run: c_n0 cached per news (DIGAT._news_cache), the news layers per pair (k3 = ffn3(c_u^(i))),
+        the user GAT stack once per behaviour; every user context reads layer j's per-behaviour nodes through share."""
+        if c_n is None:
+            c_n = self._news_ctx(w, Xn, Mn)
+        Xs = self._gat_stack(w, 'user', Xu, Au)
+        c_u, _ = self._user_ctx(w, Xs[0], Mc, ci, c_n, 0, src_index=share)
+        for i in range(self.graph_depth):
+            Xn = self._layer(w, 'news', i, Xn, An, c_u)[0]
+            c_n = self._news_ctx(w, Xn, Mn, ctx_in=c_n)
+            c_u, _ = self._user_ctx(w, Xs[i + 1], Mc, ci, c_n, i + 1, ctx_in=c_u, src_index=share)
+        return c_n, c_u
 
 
 ENCODERS = {'DIGAT': DIGAT, 'wo_SA': wo_SA, 'Seq_SA': Seq_SA, 'wo_interaction': wo_interaction,

@@ -376,7 +376,7 @@ class DIGAT(GraphEncoder):
         nu, D = Xu.shape[1], Xu.shape[2]
         B = c_n.shape[0]
         H, S = self.max_history_num, self.category_num
-        vv = linear(c_n, w['uctx_W', j], w['uctx_b', j])                          # [B, 2D or 3D]
+        vv = linear(c_n, w['uctx_W', j], w['uctx_b', j], lda=c_n.stride(0))       # [B, 2D or 3D]; c_n may be a row view
         v1, v2 = vv[:, :D], vv[:, D:2 * D]
         k3_next = vv[:, 2 * D:] if vv.shape[1] > 2 * D else None
         T = torch.empty((B, S, D), device=Xu.device, dtype=torch.float32)
@@ -633,6 +633,18 @@ class DIGAT(GraphEncoder):
         with torch.no_grad():
             return self._layer(w, 'user', index, _f32c(user_graph_embeddings, 'user_graph_embeddings'),
                                _boolc(user_graph, 'user_graph'), _f32c(news_graph_context, 'news_graph_context'))[0]
+
+    # ---- scoring interface (scoring.Scorer): what the driver gathers per pair and caches per news for _encode
+    # News-side inputs of _encode per pair: the candidate's SAG node embeddings Xn [B,n_n,D] ('graph'), its own embedding
+    # only ([B,1,D], 'first') or nothing ('none': the per-news cache holds the whole news side).
+    SCORE_NEWS_NODES = 'graph'
+
+    def _news_cache(self, w, Xn, An, Mn):
+        """The part of the scoring schedule that depends on the candidate news only, for a chunk of news (Xn [B,n_n,D],
+        An, Mn their graphs and masks).  scoring.Scorer evaluates it over the whole corpus, rebuilds it whenever the packed
+        weights change, and hands _encode the rows of each pair as c_n.  DIGAT: c_n0 [B,D] (util.py:37-44).  None = this
+        encoder caches nothing."""
+        return self._news_ctx(w, Xn, Mn)
 
     def _encode(self, w, Xn, An, Mn, Xu, Au, Mc, ci, c_n, share=None, lists=None, first_rows=None):
         """The L-layer dual-graph schedule of graphEncoders.py:180-198 on prebuilt node tensors.

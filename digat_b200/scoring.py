@@ -1,6 +1,8 @@
-"""Scoring driver over the sm_100a DIGAT encoder: the device-side part of reference util.compute_scores
-(util.py:34-69) -- SAG neighbour gather, the cached initial news-graph context c_n0, and the per-batch gathers +
-Model.inference -- with every gather done by the kernels of libdigat_sm100.so.
+"""Scoring driver over the sm_100a graph encoders (DIGAT and the five ablations): the device-side part of reference
+util.compute_scores (util.py:34-69) -- SAG neighbour gather, the cached per-news context (c_n0; util.py:39-50 dispatches
+it per encoder), and the per-batch gathers + Model.inference -- with every gather done by the kernels of libdigat_sm100.so.
+The encoder owns its scoring schedule (``_encode``), what is cached per news (``_news_cache``) and which news-side nodes
+it reads per pair (``SCORE_NEWS_NODES``).
 
 Two ways in:
 * ``score_host_batch``  takes the HOST tensors the reference DataLoader yields (util.py:56: user_title_index,
@@ -13,6 +15,8 @@ A batch is prepared in two halves (``begin_*``: launches only; ``finish_prepare`
 so that the drivers can enqueue batch k+1's first half ahead of batch k's encoder pass (see ``_pipelined``).
 Pairs are independent, so multi-GPU inference shards the pair list with no communication (``shard_range``).
 """
+import math
+
 import numpy as np
 import torch
 
@@ -29,11 +33,17 @@ def shard_range(n_items: int, rank: int, world_size: int):
 
 class Scorer:
     def __init__(self, encoder, corpus, device, build_user_graphs_on_device=False):
-        """encoder: digat_b200.graphEncoders.DIGAT on `device`; corpus: digat_b200.synth.Corpus (host numpy).
+        """encoder: one of the six graph encoders (DIGAT and the five ablations of ablation_encoders.ENCODERS) on `device`;
+        the scores are that encoder's ``inference``.  corpus: digat_b200.synth.Corpus (host numpy).
 
         build_user_graphs_on_device: derive user_graph / category mask / segment ids from the [N_beh,H] category table
         with the CUDA builder (graphs.build_user_graphs_device; bit-identical to MIND_corpus.py:143-176) instead of
         uploading the [N_beh,n_u,n_u] bool array (4.6 KB per behaviour vs 200 B)."""
+        from .ablation_encoders import ENCODERS
+        schedule = next((c for c in type(encoder).__mro__ if '_encode' in vars(c)), None)   # whose _encode would run
+        if schedule not in ENCODERS.values():
+            raise RuntimeError('Scorer: no scoring schedule for %s; supported encoders: %s'
+                               % (type(encoder).__name__, ', '.join(c.__name__ for c in ENCODERS.values())))
         self.enc = encoder.eval()
         self.dev = torch.device(device)
         if self.dev.type == 'cuda' and self.dev.index is not None and self.dev.index != torch.cuda.current_device():
@@ -59,8 +69,9 @@ class Scorer:
         self.n_news, self.D = self.table.shape
         self.n_n = self.node_id.shape[1]
         self.err = torch.zeros(1, dtype=torch.int32, device=self.dev)
-        self.c_n0 = None
+        self.c_n0 = None                                        # the encoder's per-news cache (_news_cache), or None
         self._c_n0_weights = None                               # the packed-weight generation c_n0 was computed with
+        self._first_node = None                                 # [N] int32 node_id[:, 0] (SCORE_NEWS_NODES = 'first')
 
     def _st(self):
         return torch.cuda.current_stream().cuda_stream
@@ -74,11 +85,27 @@ class Scorer:
         return out
 
     def gather_rows(self, table, idx):
+        """out[r] = table[idx[r]] for a contiguous table [N, ...] (a row is all trailing dimensions)."""
         rows = idx.numel()
-        out = torch.empty((rows, table.shape[1]), device=self.dev, dtype=torch.float32)
+        width = math.prod(table.shape[1:])
+        out = torch.empty((rows,) + tuple(table.shape[1:]), device=self.dev, dtype=torch.float32)
         _lib.call('digat_gather_rows_i32', table.data_ptr(), table.shape[0], idx.data_ptr(), out.data_ptr(),
-                  table.shape[1], rows, table.shape[1], self.err.data_ptr(), self._st())
+                  width, rows, width, self.err.data_ptr(), self._st())
         return out
+
+    def news_nodes(self, news_idx):
+        """The news-side node embeddings the encoder's scoring schedule reads per pair (its SCORE_NEWS_NODES): the SAG
+        [B,n_n,D], the candidate's own embedding [B,1,D] (SAG node 0) or None."""
+        kind = self.enc.SCORE_NEWS_NODES
+        if kind == 'graph':
+            return self.gather_sag(news_idx)
+        if kind == 'first':
+            if self._first_node is None:
+                self._first_node = self.node_id[:, 0].contiguous()
+            return self.gather_rows(self.table, self._first_node.index_select(0, news_idx.long())).view(-1, 1, self.D)
+        if kind == 'none':
+            return None
+        raise RuntimeError('%s.SCORE_NEWS_NODES must be graph, first or none (got %r)' % (type(self.enc).__name__, kind))
 
     def user_nodes(self, hist_idx):
         """[B,H] int32 history ids -> X_u [B, H+C, D] = [gathered history ; topic nodes] (util.py:65 + graphEncoders.py:191)."""
@@ -91,14 +118,21 @@ class Scorer:
         return Xu
 
     def cache_news_context(self, batch_size=1024):
-        """c_n0 for every news (util.py:37-44), in chunks of batch_size news."""
+        """The encoder's per-news cache (_news_cache) for every news, in chunks of batch_size news: c_n0 (util.py:37-44)
+        for DIGAT, Seq_SA (its sequence context) and User_graph_wo_inter; c_n^(0..L) [N, L+1, D] for the encoders with a
+        vanilla-GAT news graph; None for wo_SA."""
         w = self.enc._weights()
-        c = torch.empty((self.n_news, self.D), device=self.dev, dtype=torch.float32)
+        c = None
         with torch.no_grad():
             for lo in range(0, self.n_news, batch_size):
                 hi = min(lo + batch_size, self.n_news)
                 ids = torch.arange(lo, hi, device=self.dev, dtype=torch.int32)
-                c[lo:hi] = self.enc._news_ctx(w, self.gather_sag(ids), self.news_mask[lo:hi])
+                part = self.enc._news_cache(w, self.gather_sag(ids), self.news_graph[lo:hi], self.news_mask[lo:hi])
+                if part is None:
+                    break
+                if c is None:
+                    c = torch.empty((self.n_news,) + tuple(part.shape[1:]), device=self.dev, dtype=torch.float32)
+                c[lo:hi] = part
         self.c_n0, self._c_n0_weights = c, w
         return c
 
@@ -190,12 +224,12 @@ class Scorer:
     def score_prepared(self, prep):
         """Gathers + encoder + logits of a prepared batch: kernel launches only, no host synchronisation."""
         w = self.enc._weights()
-        if self.c_n0 is None or self._c_n0_weights is not w:     # the reference recomputes it per compute_scores call
+        if self._c_n0_weights is not w:                          # the reference recomputes it per compute_scores call
             self.cache_news_context()                            # (util.py:37-44); here: whenever the weights were repacked
         with torch.no_grad():
-            Xn = self.gather_sag(prep['news'])
+            Xn = self.news_nodes(prep['news'])
             Xu = self.user_nodes(prep['hist'])                           # one node tensor per behaviour when shared
-            c0 = self.gather_rows(self.c_n0, prep['news'])
+            c0 = None if self.c_n0 is None else self.gather_rows(self.c_n0, prep['news'])   # the pairs' cache rows
             cn, cu = self.enc._encode(w, Xn, prep['An'], prep['Mn'], Xu, prep['Au'], prep['Mc'], prep['ci'], c0,
                                       share=prep['share'],
                                       lists=(prep['prune'], prep['prune_n'], prep['seg_prune']),
